@@ -2,7 +2,7 @@
 """Benchmark of the hetero-SAGE hot path (BASELINE.json metric: message-passing edges/s over one
 train step, and top-k recs/s, at 1/2/4/8 B200 next to the CPU path).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2] [--dump-outputs DIR]
 
 A "step" is the body of the reference's ``train()`` (train_gnn.py:242-285): zero_grad -> forward
 -> pos/neg scoring + loss -> backward -> Adam step, full batch.  ``value`` = L * (2*E_eng + E_soc)
@@ -160,7 +160,32 @@ def cpu_sample_workload(w):
     return s, desc
 
 
-def run_cpu_oracle(w, steps, warmup, sample=True):
+def step_outputs(loss, model):
+    """What one train step hands its caller: the loss, and the model's parameters and gradients as the step
+    left them (host float32 / float64 arrays, keyed by the file name ``--dump-outputs`` writes them under)."""
+    import numpy as np
+    out = {"loss": np.asarray(float(loss), dtype=np.float64)}
+    for n, p in model.named_parameters():
+        out[f"param.{n}"] = p.detach().float().cpu().numpy()
+        if p.grad is not None:
+            out[f"grad.{n}"] = p.grad.detach().float().cpu().numpy()
+    return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, outputs):
+    import numpy as np
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def run_cpu_oracle(w, steps, warmup, sample=True, outputs=None):
     from oracle import sage as osage   # bench.py executes oracle/ only here: the CPU baseline
     from truth_recommendation_gnn_b200 import synth
     s, desc = cpu_sample_workload(w) if sample else (dict(w), "full size")
@@ -174,11 +199,13 @@ def run_cpu_oracle(w, steps, warmup, sample=True):
     for i in range(warmup + steps):
         neg = synth.synth_neg(s["num_posts"], s["e_eng"], i)
         t0 = time.perf_counter()
-        osage.train_step(model, opt, g.x_dict, g.edge_index_dict, g.train_edge_index,
-                         g.interaction_type_tensor, s["num_users"], s["num_posts"], neg_p=neg)
+        loss = osage.train_step(model, opt, g.x_dict, g.edge_index_dict, g.train_edge_index,
+                                g.interaction_type_tensor, s["num_users"], s["num_posts"], neg_p=neg)
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
+    if outputs is not None:
+        outputs.update(step_outputs(loss, model))
     t = sum(times) / len(times)
     mp = L * (2 * s["e_eng"] + s["e_soc"])
     return dict(value=mp / t, unit=UNIT, cores=torch.get_num_threads(), kind="port", sample=desc,
@@ -227,7 +254,10 @@ def run_reference_arm(args, w):
     if rank != 0:
         return
     torch.set_num_threads(os.cpu_count() or 1)
-    cb = run_cpu_oracle(w, args.steps, max(args.warmup, 1))
+    outputs = {} if args.dump_outputs else None
+    cb = run_cpu_oracle(w, args.steps, max(args.warmup, 1), outputs=outputs)
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": max(args.warmup, 1), "ms_per_step": cb["ms_per_step"],
@@ -253,7 +283,7 @@ def _barrier(world):
         torch.distributed.barrier()
 
 
-def gpu_train_bench(args, w, rank, world, dev, steps, warmup, e2e=True):
+def gpu_train_bench(args, w, rank, world, dev, steps, warmup, e2e=True, outputs=None):
     import truth_recommendation_gnn_b200 as trg
     from truth_recommendation_gnn_b200 import _lib, synth
     from truth_recommendation_gnn_b200 import dist as tdist
@@ -322,21 +352,25 @@ def gpu_train_bench(args, w, rank, world, dev, steps, warmup, e2e=True):
     _barrier(world); torch.cuda.synchronize()
     n0 = _lib.launch_count()
     clocks.start()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    t_host0 = time.perf_counter()
-    loss = None
-    for i in range(steps):
-        loss = step(i, False)
-    host_ms = (time.perf_counter() - t_host0) * 1e3 / steps     # CPU time to ENQUEUE one step
-    e1.record()
-    torch.cuda.synchronize(); _barrier(world)
+    try:
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        t_host0 = time.perf_counter()
+        loss = None
+        for i in range(steps):
+            loss = step(i, False)
+        host_ms = (time.perf_counter() - t_host0) * 1e3 / steps     # CPU time to ENQUEUE one step
+        e1.record()
+        torch.cuda.synchronize(); _barrier(world)
+    finally:
+        clk = clocks.stop()       # also on failure: the sampler must not outlive the job
     loss = float(loss)        # now: a graphed step returns its static loss tensor, which later replays overwrite
-    clk = clocks.stop()
     n1 = _lib.launch_count()
     _lib.PROF.enabled = False
     ms = e0.elapsed_time(e1) / steps
     prof = _lib.PROF.summary()
+    if outputs is not None:       # before the e2e leg, whose steps train the model further
+        outputs.update(step_outputs(loss, model))
 
     # ---- timed region 2: end to end through the public API with host buffers ----
     ms_e2e = None
@@ -403,7 +437,7 @@ def sub_line(name, w, r, world, steps):
             "gpu_launches": r["launches"], "host_enqueue_ms_per_step": round(r["host_ms"], 3)}
 
 
-def gpu_topk_bench(dev, rank, world, iters=3):
+def gpu_topk_bench(dev, rank, world, iters=3, outputs=None):
     """Secondary metric: top-k recs/s -- inference.py:427-428 batched, BASELINE config 5 (score all 50M posts per
     user batch of 4096, top-100; bf16 in, fp32 accumulate; tcgen05 + warp-level select).  N > 1: the catalogue is
     sharded by post-id range (each rank holds 50M / N rows), queries replicated, per-shard lists all-gathered and
@@ -429,10 +463,13 @@ def gpu_topk_bench(dev, rank, world, iters=3):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(iters):
-        call(q)
+        v, i = call(q)
     e1.record()
     torch.cuda.synchronize(); _barrier(world)
     ms = e0.elapsed_time(e1) / iters
+    if outputs is not None:
+        outputs["topk.values"] = v.float().cpu().numpy()
+        outputs["topk.ids"] = i.cpu().double().numpy()      # post ids < 2^53: exact in float64
     # end to end: the query batch comes from pinned host memory, ids + scores go back to the host
     v, i = call(q_host.to(dev, non_blocking=True))     # untimed: first-use host staging buffers
     v, i = v.cpu(), i.cpu()
@@ -491,7 +528,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-topk", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline only: skip cfg1 / cfg3 / cfg4 / verify")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, parameters and gradients after the "
+                         "step; the top-k leg's scores and ids) as DIR/<name>.npy, to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -512,7 +554,8 @@ def main():
     if world > 1:
         torch.distributed.init_process_group("nccl", device_id=dev)
 
-    r = gpu_train_bench(args, w, rank, world, dev, args.steps, args.warmup)
+    outputs = {} if args.dump_outputs and rank == 0 else None
+    r = gpu_train_bench(args, w, rank, world, dev, args.steps, args.warmup, outputs=outputs)
     if rank == 0:
         print(f"[bench] headline {args.workload} x{world}: {r['ms']:.3f} ms/step, e2e {r['ms_e2e']:.3f}, "
               f"kernels {({k: round(v['ms'] / args.steps, 3) for k, v in sorted(r['prof'].items())})}",
@@ -564,8 +607,10 @@ def main():
             leg("cfg4", lambda: (w4, gpu_train_bench(args, w4, rank, world, dev, min(args.steps, 5), 3, e2e=False), min(args.steps, 5)),
                 limit=300.0)
     if not args.no_topk:
-        leg("topk", lambda: gpu_topk_bench(dev, rank, world))
+        leg("topk", lambda: gpu_topk_bench(dev, rank, world, outputs=outputs))
 
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(build_line(final=True)))
     if world > 1:

@@ -462,3 +462,51 @@ def test_train_step_cuda_graph_matches_eager(dev, layers):
     assert losses["eager"] == pytest.approx(losses["graph"], rel=1e-6)
     for a, b in zip(weights["eager"], weights["graph"]):
         assert torch.allclose(a, b, rtol=1e-5, atol=1e-7)
+
+
+def test_bench_dumps_the_last_timed_step(dev, tmp_path):
+    """``bench.py --dump-outputs DIR`` writes what its last timed step computed: after 3 warm-up and ``--steps 2``
+    timed steps on the tiny workload, the loss, parameters and gradients equal those of the same 5 steps run
+    here; the top-k leg's scores and ids come out as sorted, in-range rows."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, "bench.py", "--workload", "tiny", "--steps", "2", "--warmup", "3",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, cwd=root, timeout=600)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and "topk" in line
+    out = {f[:-len(".npy")]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    assert float(out["loss"]) == line["loss"]
+
+    sys.path.insert(0, root)
+    import bench
+    w = bench.WORKLOADS["tiny"]
+    U, P, Ee, Es, H, L = w["num_users"], w["num_posts"], w["e_eng"], w["e_soc"], w["hidden"], w["layers"]
+    g = synth.synth_graph(U, P, Ee, Es, H, seed=0, device=dev)
+    model = _gpu_model(H, L, synth.init_state_dict(H, H, L), dev)
+    opt = torch.optim.Adam(model.parameters(), lr=1e-3)
+    for i in (0, 1, 2, 0, 1):          # bench.py cycles through 4 negative draws: warm-up 0..2, timed 0..1
+        loss = trg.train_step(model, opt, g.x_dict, g.edge_index_dict, g.train_edge_index,
+                              g.interaction_type_tensor, U, P, neg_p=synth.synth_neg(P, Ee, i, device=dev))
+    assert float(out["loss"]) == pytest.approx(loss, rel=1e-6)
+    names = [n for n, _ in model.named_parameters()]
+    assert sorted(out) == sorted(["loss", "topk.values", "topk.ids"] + [f"{k}.{n}" for k in ("param", "grad")
+                                                                         for n in names])
+    for n, p in model.named_parameters():
+        assert torch.allclose(torch.from_numpy(out[f"param.{n}"]), p.detach().cpu(), rtol=1e-5, atol=1e-7), n
+        assert_close(torch.from_numpy(out[f"grad.{n}"]), p.grad.cpu(), TOL_F32, f"grad {n}")
+
+    vals, ids = out["topk.values"], out["topk.ids"]
+    t = bench.TOPK
+    assert vals.shape == ids.shape == (t["batch"], t["k"])
+    assert (np.diff(vals, axis=1) <= 0).all()
+    assert (ids == np.round(ids)).all() and ids.min() >= 0 and ids.max() < t["n_post"]
+    assert all(len(set(row)) == t["k"] for row in ids[:64].tolist())

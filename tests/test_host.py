@@ -186,17 +186,21 @@ def test_negative_share_capacity_covers_randint_modulo_bias():
     assert sh.neg_capacity() > 100_132_949
 
 
-def test_bench_reference_arm_line_contract():
-    """``bench.py --impl reference`` (the driver runs it next to the GPU arm): one JSON line on stdout with the
+def test_bench_reference_arm_line_contract(tmp_path):
+    """``bench.py --impl reference`` (run next to the GPU arm): one JSON line on stdout with the
     contract's keys, the SAME ``config`` object the GPU arm prints for that workload, and a ``cpu_baseline``
-    describing the run.  Runs the tiny workload on the CPU oracle (no GPU involved)."""
+    describing the run; ``--dump-outputs`` writes the last timed step's loss, parameters and gradients.  Runs
+    the tiny workload on the CPU oracle (no GPU involved)."""
     import json
     import os
     import subprocess
     import sys
+
+    import numpy as np
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     r = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--workload", "tiny", "--steps", "2",
-                        "--warmup", "1", "--no-extras"], capture_output=True, text=True, cwd=root, timeout=600)
+                        "--warmup", "1", "--no-extras", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, cwd=root, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -211,6 +215,15 @@ def test_bench_reference_arm_line_contract():
     import bench
     assert d["config"] == bench.config_of("tiny", bench.WORKLOADS["tiny"])      # identical in both arms
     assert d["value"] > 0 and d["steps"] == 2
+    w = bench.WORKLOADS["tiny"]
+    sd = synth.init_state_dict(w["hidden"], w["hidden"], w["layers"])
+    out = {f[:-len(".npy")]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert sorted(out) == sorted(["loss"] + [f"{k}.{n}" for k in ("param", "grad") for n in sd])
+    assert out["loss"].dtype == np.float64 and out["loss"].shape == () and np.isfinite(out["loss"])
+    for n, v in sd.items():
+        p, gr = out[f"param.{n}"], out[f"grad.{n}"]
+        assert p.dtype == gr.dtype == np.float32 and p.shape == gr.shape == tuple(v.shape)
+        assert np.isfinite(gr).all() and not np.array_equal(p, v.numpy()), n     # the steps moved every tensor
 
 
 def test_bench_refuses_to_run_the_product_without_a_gpu():
