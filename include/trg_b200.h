@@ -243,6 +243,24 @@ int trg_score_topk(const void* q /* [B, H] */, const void* cat /* [P, H] */,
                    int64_t n_query, int64_t n_cat, int32_t hidden, int dtype, int32_t k,
                    int64_t id_offset, float* vals_out /* [B, k_out] */, int64_t* ids_out /* [B, k_out] */,
                    void* workspace, size_t workspace_bytes, void* stream);
+/* trg_score_topk with a per-query list of posts that must not be returned (e.g. the posts a user has
+ * already engaged with).  The exclusion index is a CSR over "exclusion rows":
+ *   excl_rowptr int32[R+1]; excl_ids int32[nnz] holding GLOBAL post ids (the id space of ids_out:
+ *   local + id_offset), ascending within each row.  Duplicates are allowed, and so are ids outside the
+ *   catalogue or shard (they never match).
+ * Query b uses exclusion row query_rows[b], or row b when query_rows is NULL.  The result of query b is
+ * the top k_out = min(k, n_cat) posts of the catalogue with that row's ids removed, under the same total
+ * order (score desc, id asc).  A row with fewer than k_out admissible posts is padded at its tail with
+ * (-inf, -1); the output stays [B, k_out].  An empty exclusion row gives exactly trg_score_topk's result.
+ * excl_rowptr == NULL means no exclusions (then this is trg_score_topk); excl_ids must be non-NULL when
+ * excl_rowptr is given.  The index is read on the device only (no host sync).  Same workspace as
+ * trg_score_topk (trg_score_topk_workspace_bytes). */
+int trg_score_topk_excluding(const void* q /* [B, H] */, const void* cat /* [P, H] */,
+                             int64_t n_query, int64_t n_cat, int32_t hidden, int dtype, int32_t k,
+                             int64_t id_offset, const int32_t* excl_rowptr /* [R+1] */,
+                             const int32_t* excl_ids /* [nnz] */, const int64_t* query_rows /* [B], nullable */,
+                             float* vals_out /* [B, k_out] */, int64_t* ids_out /* [B, k_out] */,
+                             void* workspace, size_t workspace_bytes, void* stream);
 /* Merge n_lists per-row sorted (vals, ids) lists of length k_in into the top k_out. */
 int trg_topk_merge(const float* vals_in /* [B, n_lists*k_in] */, const int64_t* ids_in,
                    int64_t n_query, int32_t n_lists, int32_t k_in, int32_t k_out,

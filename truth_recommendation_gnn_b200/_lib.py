@@ -67,6 +67,8 @@ SIGNATURES = {
                                         _vp, _sz, _vp]),
     "trg_score_topk_workspace_bytes": (_sz, [_i64, _i64, _i32, _i32]),
     "trg_score_topk": (_int, [_vp, _vp, _i64, _i64, _i32, _int, _i32, _i64, _vp, _vp, _vp, _sz, _vp]),
+    "trg_score_topk_excluding": (_int, [_vp, _vp, _i64, _i64, _i32, _int, _i32, _i64, _vp, _vp, _vp, _vp, _vp,
+                                        _vp, _sz, _vp]),
     "trg_topk_merge": (_int, [_vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp]),
 }
 

@@ -12,6 +12,7 @@
 // shapes); the bf16 tcgen05 form for 50M-post catalogues is score_topk_tc.cu.
 #include <algorithm>
 #include <cfloat>
+#include <climits>
 
 #include "common.cuh"
 
@@ -78,9 +79,25 @@ struct ScoreArgs {
   int64_t n_query, n_cat, id_offset;
   int hidden, k, n_splits;
   int64_t tiles_per_split;
+  // exclusion index (EXCL instantiation only; appended so that the fields above keep their offsets)
+  const int32_t* excl_rowptr;   // [R + 1]
+  const int32_t* excl_ids;      // [nnz] global post ids, ascending within a row
+  const int64_t* query_rows;    // [B] exclusion row of each query, nullable (= the query's own row)
 };
 
+// first index in ids[lo, hi) (ascending) whose value is >= v
+__device__ __forceinline__ int excl_lower_bound(const int32_t* __restrict__ ids, int lo, int hi, long long v) {
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if ((long long)__ldg(ids + mid) < v) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
 // dynamic smem: Qs[kBQ][ld] | Ps[kBP][ld] | lv[kBQ][kMaxK] | li[kBQ][kMaxK]
+// EXCL: a post of the query row's exclusion list never passes the filter, so the lists (and thresholds)
+// only ever hold admissible posts.  The test runs only on lanes that already pass the threshold.
+template <bool EXCL>
 __global__ void __launch_bounds__(kThreads) score_topk_f32(const ScoreArgs a) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int H = a.hidden, ld = H + 4;
@@ -106,8 +123,37 @@ __global__ void __launch_bounds__(kThreads) score_topk_f32(const ScoreArgs a) {
   const int64_t tile0 = (int64_t)split * a.tiles_per_split;
   const int64_t n_tiles = ceil_div<int64_t>(a.n_cat, kBP);
   const int64_t tile1 = min(tile0 + a.tiles_per_split, n_tiles);
+  // EXCL: the part of each of the warp's 4 rows' exclusion lists inside this split's id range, as a cursor
+  // [ex_lo, ex_hi) that follows the tiles (ascending ids) and the id at the cursor, ex_v (LLONG_MAX: none left)
+  int ex_lo[4] = {0, 0, 0, 0}, ex_hi[4] = {0, 0, 0, 0};
+  long long ex_v[4] = {LLONG_MAX, LLONG_MAX, LLONG_MAX, LLONG_MAX};
+  if constexpr (EXCL) {
+    int lo = 0, hi = 0;
+    const int64_t qi = q0 + 4 * w + lane;
+    if (lane < 4 && qi < a.n_query) {
+      const int64_t er = a.query_rows ? a.query_rows[qi] : qi;
+      const int b0 = __ldg(a.excl_rowptr + er), b1 = __ldg(a.excl_rowptr + er + 1);
+      lo = excl_lower_bound(a.excl_ids, b0, b1, a.id_offset + tile0 * kBP);
+      hi = excl_lower_bound(a.excl_ids, lo, b1, a.id_offset + tile1 * kBP);
+    }
+#pragma unroll
+    for (int x = 0; x < 4; ++x) {
+      ex_lo[x] = __shfl_sync(0xffffffffu, lo, x);
+      ex_hi[x] = __shfl_sync(0xffffffffu, hi, x);
+      if (ex_lo[x] < ex_hi[x]) ex_v[x] = __ldg(a.excl_ids + ex_lo[x]);
+    }
+  }
   for (int64_t tile = tile0; tile < tile1; ++tile) {
     const int64_t p0 = tile * kBP;
+    if constexpr (EXCL) {
+      // move each row's cursor to its first excluded id >= this tile's first post (one load per excluded id)
+#pragma unroll
+      for (int x = 0; x < 4; ++x)
+        while (ex_v[x] < a.id_offset + p0) {
+          ++ex_lo[x];
+          ex_v[x] = ex_lo[x] < ex_hi[x] ? (long long)__ldg(a.excl_ids + ex_lo[x]) : LLONG_MAX;
+        }
+    }
     __syncthreads();  // previous tile's Ps fully consumed (also orders the Qs fill)
     for (int i = tid; i < kBP * hv; i += kThreads) {
       const int r = i / hv, c = i % hv;
@@ -148,7 +194,21 @@ __global__ void __launch_bounds__(kThreads) score_topk_f32(const ScoreArgs a) {
         const int64_t pid = p0 + lane + 32 * y;
         const float s = acc[x][y];
         const bool valid = pid < a.n_cat;
-        unsigned cand = __ballot_sync(0xffffffffu, valid && (!full[x] || s > thr[x]));
+        bool pass = valid && (!full[x] || s > thr[x]);
+        if constexpr (EXCL) {
+          // most tiles hold none of the row's excluded ids (ex_v past the tile): a register test
+          const long long gid = a.id_offset + pid;
+          if (pass && ex_v[x] < a.id_offset + p0 + kBP) {
+            if (gid == ex_v[x]) {
+              pass = false;
+            } else if (gid > ex_v[x]) {
+              const int at = excl_lower_bound(a.excl_ids, ex_lo[x] + 1, ex_hi[x], gid);
+              pass = !(at < ex_hi[x] && (long long)__ldg(a.excl_ids + at) == gid);
+            }
+          }
+        }
+        // excluded lanes stay out of `cand`: the re-filter below only ever clears bits
+        unsigned cand = __ballot_sync(0xffffffffu, pass);
         while (cand) {
           const int l = __ffs(cand) - 1;
           const float cs = __shfl_sync(0xffffffffu, s, l);
@@ -237,9 +297,20 @@ namespace tc {
 bool score_tc_eligible(int hidden, int dtype, int k);
 size_t score_tc_workspace_bytes(int64_t n_query, int64_t n_cat, int hidden, int k);
 int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat, int hidden, int k,
-                  int64_t id_offset, float* vals_out, int64_t* ids_out, void* ws, size_t ws_bytes,
+                  int64_t id_offset, const int32_t* excl_rowptr, const int32_t* excl_ids,
+                  const int64_t* query_rows, float* vals_out, int64_t* ids_out, void* ws, size_t ws_bytes,
                   cudaStream_t st);
 }  // namespace tc
+
+namespace {
+template <bool EXCL>
+int launch_f32(const ScoreArgs& a, dim3 grid, size_t smem, cudaStream_t st) {
+  static SmemAttrState attr;
+  TRG_CUDA(ensure_dyn_smem(score_topk_f32<EXCL>, (int)smem, attr));
+  score_topk_f32<EXCL><<<grid, kThreads, smem, st>>>(a);
+  return TRG_OK;
+}
+}  // namespace
 }  // namespace trg
 
 using namespace trg;
@@ -276,34 +347,36 @@ extern "C" int trg_topk_merge(const float* vals_in, const int64_t* ids_in, int64
   return TRG_OK;
 }
 
-extern "C" int trg_score_topk(const void* q, const void* cat, int64_t n_query, int64_t n_cat,
-                              int32_t hidden, int dtype, int32_t k, int64_t id_offset,
-                              float* vals_out, int64_t* ids_out, void* workspace,
-                              size_t workspace_bytes, void* stream) {
+// trg_score_topk and trg_score_topk_excluding: excl_rowptr == NULL means no exclusions (the shipped kernels)
+static int score_topk_impl(const char* fn, const void* q, const void* cat, int64_t n_query, int64_t n_cat,
+                           int32_t hidden, int dtype, int32_t k, int64_t id_offset, const int32_t* excl_rowptr,
+                           const int32_t* excl_ids, const int64_t* query_rows, float* vals_out, int64_t* ids_out,
+                           void* workspace, size_t workspace_bytes, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  TRG_CHECK_ARG(n_query >= 0 && n_cat >= 0 && k > 0, "trg_score_topk: bad sizes");
+  TRG_CHECK_ARG(n_query >= 0 && n_cat >= 0 && k > 0, "%s: bad sizes", fn);
   if (n_query == 0 || n_cat == 0) return TRG_OK;
-  TRG_CHECK_ARG(q && cat && vals_out && ids_out, "trg_score_topk: NULL pointer");
-  TRG_CHECK_ARG(((uintptr_t)q | (uintptr_t)cat) % 16 == 0, "trg_score_topk: tables must be 16-byte aligned");
+  TRG_CHECK_ARG(q && cat && vals_out && ids_out, "%s: NULL pointer", fn);
+  TRG_CHECK_ARG(((uintptr_t)q | (uintptr_t)cat) % 16 == 0, "%s: tables must be 16-byte aligned", fn);
+  TRG_CHECK_ARG(!excl_rowptr || excl_ids, "%s: excl_ids must be non-NULL when excl_rowptr is given", fn);
   const int kk = (int)std::min<int64_t>(k, n_cat);
-  TRG_CHECK_ARG(kk <= kMaxK, "trg_score_topk: k=%d > %d is not supported", kk, kMaxK);
+  TRG_CHECK_ARG(kk <= kMaxK, "%s: k=%d > %d is not supported", fn, kk, kMaxK);
   if (dtype == TRG_BF16) {
     if (!tc::score_tc_eligible(hidden, dtype, kk)) {
-      set_error("trg_score_topk(bf16): hidden=%d k=%d unsupported: hidden must be in {64,128,192,256}, k <= 128, and the query block (256*hidden B) + the per-row lists (1 KiB*k) + two catalogue stages must fit in 227 KiB of shared memory", hidden, kk);
+      set_error("%s(bf16): hidden=%d k=%d unsupported: hidden must be in {64,128,192,256}, k <= 128, and the query block (256*hidden B) + the per-row lists (1 KiB*k) + two catalogue stages must fit in 227 KiB of shared memory", fn, hidden, kk);
       return TRG_E_UNSUPPORTED;
     }
-    return tc::score_topk_tc(q, cat, n_query, n_cat, hidden, kk, id_offset, vals_out, ids_out, workspace,
-                             workspace_bytes, st);
+    return tc::score_topk_tc(q, cat, n_query, n_cat, hidden, kk, id_offset, excl_rowptr, excl_ids, query_rows,
+                             vals_out, ids_out, workspace, workspace_bytes, st);
   }
   if (dtype != TRG_F32) {
-    set_error("trg_score_topk: unknown dtype %d", dtype);
+    set_error("%s: unknown dtype %d", fn, dtype);
     return TRG_E_ARG;
   }
   TRG_CHECK_ARG(hidden > 0 && hidden % 4 == 0 && hidden <= 256,
-                "trg_score_topk(fp32): hidden=%d must be a multiple of 4 and <= 256", hidden);
+                "%s(fp32): hidden=%d must be a multiple of 4 and <= 256", fn, hidden);
   const size_t need = trg_score_topk_workspace_bytes(n_query, n_cat, hidden, k);
   if (workspace == nullptr || workspace_bytes < need) {
-    set_error("trg_score_topk: workspace %zu < required %zu", workspace_bytes, need);
+    set_error("%s: workspace %zu < required %zu", fn, workspace_bytes, need);
     return TRG_E_WORKSPACE;
   }
   ScoreArgs a{};
@@ -313,13 +386,30 @@ extern "C" int trg_score_topk(const void* q, const void* cat, int64_t n_query, i
   a.part_vals = reinterpret_cast<float*>(workspace);
   a.part_ids = reinterpret_cast<long long*>(reinterpret_cast<char*>(workspace) +
                                             align_up((size_t)n_query * a.n_splits * kk * 4, 256));
+  a.excl_rowptr = excl_rowptr; a.excl_ids = excl_ids; a.query_rows = query_rows;
   const size_t smem = score_smem_bytes(hidden);
-  static SmemAttrState attr;
-  TRG_CUDA(ensure_dyn_smem(score_topk_f32, (int)smem, attr));
   dim3 grid((unsigned)ceil_div<int64_t>(n_query, kBQ), (unsigned)a.n_splits);
-  score_topk_f32<<<grid, kThreads, smem, st>>>(a);
+  const int rc = excl_rowptr ? launch_f32<true>(a, grid, smem, st) : launch_f32<false>(a, grid, smem, st);
+  if (rc) return rc;
   count_launch();
   TRG_LAUNCH_OK();
   return trg_topk_merge(a.part_vals, (const int64_t*)a.part_ids, n_query, a.n_splits, kk, kk,
                         vals_out, ids_out, stream);
+}
+
+extern "C" int trg_score_topk(const void* q, const void* cat, int64_t n_query, int64_t n_cat,
+                              int32_t hidden, int dtype, int32_t k, int64_t id_offset,
+                              float* vals_out, int64_t* ids_out, void* workspace,
+                              size_t workspace_bytes, void* stream) {
+  return score_topk_impl("trg_score_topk", q, cat, n_query, n_cat, hidden, dtype, k, id_offset, nullptr, nullptr,
+                         nullptr, vals_out, ids_out, workspace, workspace_bytes, stream);
+}
+
+extern "C" int trg_score_topk_excluding(const void* q, const void* cat, int64_t n_query, int64_t n_cat,
+                                        int32_t hidden, int dtype, int32_t k, int64_t id_offset,
+                                        const int32_t* excl_rowptr, const int32_t* excl_ids,
+                                        const int64_t* query_rows, float* vals_out, int64_t* ids_out,
+                                        void* workspace, size_t workspace_bytes, void* stream) {
+  return score_topk_impl("trg_score_topk_excluding", q, cat, n_query, n_cat, hidden, dtype, k, id_offset,
+                         excl_rowptr, excl_ids, query_rows, vals_out, ids_out, workspace, workspace_bytes, stream);
 }

@@ -50,6 +50,10 @@ struct ScoreTcParams {
   int* locks;                 // [B] one lock per query row's global list
   float* out_vals;            // [B][k] the rows' global top-K lists (= the result), merged into by every item
   long long* out_ids;         // [B][k]
+  // exclusion index (EXCL instantiations only; appended so that the fields above keep their offsets)
+  const int* excl_rowptr;     // [R + 1]
+  const int* excl_ids;        // [nnz] global post ids, ascending within a row
+  const long long* query_rows;   // [B] exclusion row of each query, nullable (= the query's own row)
 };
 
 // Ablation / cycle-accounting switches alter results; they exist only in -DTRG_DEBUG builds.
@@ -73,6 +77,14 @@ __device__ __forceinline__ uint32_t lds32(uint32_t a) {
 }
 __device__ __forceinline__ void sts32(uint32_t a, uint32_t v) {
   asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory");
+}
+// first index in ids[lo, hi) (ascending) whose value is >= v
+__device__ __forceinline__ int excl_lower_bound(const int* __restrict__ ids, int lo, int hi, long long v) {
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if ((long long)__ldg(ids + mid) < v) lo = mid + 1; else hi = mid;
+  }
+  return lo;
 }
 // a ranks before b under (score desc, id asc)
 __device__ __forceinline__ bool ranks_before(float sa, uint32_t ia, float sb, uint32_t ib) {
@@ -305,7 +317,11 @@ __device__ __forceinline__ float merge_into_global(const ScoreTcParams& p, long 
   return kth_key == (int)0x80000000 ? -INFINITY : key_float(kth_key);
 }
 
-template <int NS>
+// EXCL: the helper warps' exact test also rejects the posts of each query row's exclusion list, so no
+// excluded post ever enters a list -- per-item lists, flushed global lists, row_thr and thr_shared then only
+// ever hold admissible posts, and every threshold below stays the exact K-th best of what may be returned.
+// The scan warps' filter (max against those thresholds) remains a superset test and is unchanged.
+template <int NS, bool EXCL>
 __global__ void __launch_bounds__(512, 1)
     score_topk_tc3_kernel(const __grid_constant__ ScoreTcParams p, int n_stages) {
   constexpr int N = kTileN2;
@@ -545,6 +561,8 @@ __global__ void __launch_bounds__(512, 1)
     long long idbase = 0;   // global id of the current item's first post
     int cnt = 0;     // lane l: entries in the queue of row 32 wq + l
     int m = 0;       // lane l: entries in the list of row 32 wq + l
+    int ex_lo = 0, ex_hi = 0;   // EXCL, lane l: the part of row 32 wq + l's exclusion list inside this item's chunk
+    uint32_t ex_first = 0;      //              and its first id (relative to idbase)
     // merge the last `n_c` (<= 32) queue entries of row L into its list (TMEM lane L, staged through scratch)
     auto merge_row = [&](int L, int n_c, int q_off) {
       const int row = wq * 32 + L;
@@ -630,6 +648,13 @@ __global__ void __launch_bounds__(512, 1)
       const int nvalid = (int)hdr.z;
       const int row = wq * 32 + L;
       const float tg = *reinterpret_cast<volatile float*>(row_tg + row);
+      int x_lo = 0, x_hi = 0;
+      uint32_t x_first = 0;
+      if constexpr (EXCL) {
+        x_lo = __shfl_sync(0xffffffffu, ex_lo, L);
+        x_hi = __shfl_sync(0xffffffffu, ex_hi, L);
+        x_first = __shfl_sync(0xffffffffu, ex_first, L);
+      }
 #pragma unroll 1
       for (int i = 0; i < kHalfN3 / 32; ++i) {
         // the row's exact K-th best (it may have moved in the previous sub-step's merge)
@@ -639,7 +664,20 @@ __global__ void __launch_bounds__(512, 1)
         const int j = i * 32 + lane;
         const float s = __uint_as_float(lds32(sa + (uint32_t)(j * 4)));
         const uint32_t id = base_idx + (uint32_t)j;
-        const bool pass = j < nvalid && s >= tg && (s > thr || (s == thr && id < ti));
+        bool pass = j < nvalid && s >= tg && (s > thr || (s == thr && id < ti));
+        if constexpr (EXCL) {
+          // the chunk's part of the row's exclusion list is usually empty or one entry, whose id is in a
+          // register: a search in global memory only past it, and only by lanes that already pass the exact test
+          if (pass && x_lo < x_hi) {
+            if (id == x_first) {
+              pass = false;
+            } else if (id > x_first && x_hi - x_lo > 1) {
+              const long long gid = idbase + (long long)id;
+              const int at = excl_lower_bound(p.excl_ids, x_lo + 1, x_hi, gid);
+              pass = !(at < x_hi && (long long)__ldg(p.excl_ids + at) == gid);
+            }
+          }
+        }
         const unsigned pm = __ballot_sync(0xffffffffu, pass);
         if (pm) {
           const int n = __popc(pm);
@@ -667,6 +705,17 @@ __global__ void __launch_bounds__(512, 1)
     while (next_segment(p, n_tiles_total, n_qb, item, sg)) {
       q0 = sg.qb * kQRows;
       idbase = p.id_offset + sg.tile0 * N;
+      if constexpr (EXCL) {
+        const long long gq = q0 + wq * 32 + lane;
+        ex_lo = ex_hi = 0;
+        if (gq < p.n_query) {
+          const long long er = p.query_rows ? p.query_rows[gq] : gq;
+          const int b0 = __ldg(p.excl_rowptr + er), b1 = __ldg(p.excl_rowptr + er + 1);
+          ex_lo = excl_lower_bound(p.excl_ids, b0, b1, idbase);
+          ex_hi = excl_lower_bound(p.excl_ids, ex_lo, b1, idbase + p.tiles_per_split * N);
+          if (ex_lo < ex_hi) ex_first = (uint32_t)(__ldg(p.excl_ids + ex_lo) - idbase);
+        }
+      }
       for (;;) {
         // poll the two rings of this quarter (SCAN A: ring wq, SCAN B: ring 4 + wq)
         int h[2] = {0, 0}, dn[2] = {0, 0};
@@ -821,16 +870,23 @@ __global__ void init_lists(float* vals, long long* ids, long long n, int* thr, i
   }
 }
 
-template <int NS>
+// with exclusions a row may have fewer than K admissible posts: its list keeps pads, reported as id -1
+__global__ void pads_to_minus_one(long long* ids, long long n) {
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    if (ids[i] == kPadIdTc) ids[i] = -1;
+}
+
+template <int NS, bool EXCL>
 static int launch_score3(const ScoreTcParams& p, int grid, int smem, int n_stages, cudaStream_t st) {
   static SmemAttrState attr;
-  TRG_CUDA(ensure_dyn_smem(score_topk_tc3_kernel<NS>, smem, attr));
-  score_topk_tc3_kernel<NS><<<grid, 512, smem, st>>>(p, n_stages);
+  TRG_CUDA(ensure_dyn_smem(score_topk_tc3_kernel<NS, EXCL>, smem, attr));
+  score_topk_tc3_kernel<NS, EXCL><<<grid, 512, smem, st>>>(p, n_stages);
   return TRG_OK;
 }
 
 int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat, int hidden, int k,
-                  int64_t id_offset, float* vals_out, int64_t* ids_out, void* ws, size_t ws_bytes,
+                  int64_t id_offset, const int32_t* excl_rowptr, const int32_t* excl_ids,
+                  const int64_t* query_rows, float* vals_out, int64_t* ids_out, void* ws, size_t ws_bytes,
                   cudaStream_t st) {
   const size_t need = score_tc_workspace_bytes(n_query, n_cat, hidden, k);
   if (!ws || ws_bytes < need) {
@@ -854,14 +910,30 @@ int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat
   p.locks = reinterpret_cast<int*>(reinterpret_cast<char*>(ws) + align_up((size_t)n_query * 4, 256));
   p.out_vals = vals_out;
   p.out_ids = reinterpret_cast<long long*>(ids_out);
+  p.excl_rowptr = excl_rowptr;
+  p.excl_ids = excl_ids;
+  p.query_rows = reinterpret_cast<const long long*>(query_rows);
+  const bool excl = excl_rowptr != nullptr;
   const long long n_out = std::max<long long>((long long)n_query * k, n_query);
   init_lists<<<(unsigned)std::min<long long>(2048, (n_out + 255) / 256), 256, 0, st>>>(
       p.out_vals, p.out_ids, (long long)n_query * k, p.thr_shared, p.locks, n_query);
   count_launch();
-  rc = cfg.ns == kTileN2 ? launch_score3<kTileN2>(p, grid, cfg.smem, cfg.stages, st)
-                         : launch_score3<kTileN2 / 2>(p, grid, cfg.smem, cfg.stages, st);
+  // the EXCL = false instantiations come first: the compiler then emits them instruction for instruction as
+  // the kernel was before exclusions existed (instantiated after the EXCL ones, the NS = 64 form came out
+  // with a different register assignment)
+  if (!excl)
+    rc = cfg.ns == kTileN2 ? launch_score3<kTileN2, false>(p, grid, cfg.smem, cfg.stages, st)
+                           : launch_score3<kTileN2 / 2, false>(p, grid, cfg.smem, cfg.stages, st);
+  else
+    rc = cfg.ns == kTileN2 ? launch_score3<kTileN2, true>(p, grid, cfg.smem, cfg.stages, st)
+                           : launch_score3<kTileN2 / 2, true>(p, grid, cfg.smem, cfg.stages, st);
   if (rc) return rc;
   count_launch();
+  if (excl) {
+    const long long n = (long long)n_query * k;
+    pads_to_minus_one<<<(unsigned)std::min<long long>(2048, (n + 255) / 256), 256, 0, st>>>(p.out_ids, n);
+    count_launch();
+  }
   TRG_LAUNCH_OK();
   return TRG_OK;
 }

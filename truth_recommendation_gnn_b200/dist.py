@@ -378,22 +378,31 @@ def train_step_sharded(model, optimizer, shard: ShardedGraph, neg_p_global=None,
 
 
 @torch.no_grad()
-def recommend_sharded(q, cat_local, k, id_offset, score_topk_fn=None, merge_fn=None):
+def recommend_sharded(q, cat_local, k, id_offset, score_topk_fn=None, merge_fn=None, exclude=None, rows=None):
     """Catalogue sharded by post-id range: local score + top-k, all-gather of the per-shard
-    ``(values, global ids)``, merge under (score desc, id asc) == the unsharded result."""
+    ``(values, global ids)``, merge under (score desc, id asc) == the unsharded result.
+    ``exclude`` / ``rows`` (see ``score_topk``): every rank passes the same index, since its ids are
+    global; rows short of admissible posts end in ``(-inf, -1)`` pads, as unsharded."""
     from . import functional as Fn
     score_topk_fn = score_topk_fn or Fn.score_topk
     merge_fn = merge_fn or Fn.topk_merge
     world = dist.get_world_size()
-    vals, ids = score_topk_fn(q, cat_local, k, id_offset)
+    if exclude is None and rows is None:
+        vals, ids = score_topk_fn(q, cat_local, k, id_offset)
+    else:
+        vals, ids = score_topk_fn(q, cat_local, k, id_offset, exclude=exclude, rows=rows)
     kk = vals.size(1)
     if world == 1:
         return vals, ids
+    pad_id = torch.iinfo(torch.int64).max
+    if exclude is not None:
+        # the merge treats only id INT64_MAX as padding
+        ids = torch.where(ids < 0, torch.full_like(ids, pad_id), ids)
     # shards may hold fewer than k posts: pad lists so every rank contributes k columns
     if kk < k:
         pad = k - kk
         vals = torch.cat([vals, torch.full((vals.size(0), pad), float("-inf"), device=vals.device)], 1)
-        ids = torch.cat([ids, torch.full((ids.size(0), pad), torch.iinfo(torch.int64).max, device=ids.device)], 1)
+        ids = torch.cat([ids, torch.full((ids.size(0), pad), pad_id, device=ids.device)], 1)
     b = vals.size(0)
     av = torch.empty(world * b, k, dtype=vals.dtype, device=vals.device)
     ai = torch.empty(world * b, k, dtype=ids.dtype, device=ids.device)

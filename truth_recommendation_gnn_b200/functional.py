@@ -526,9 +526,14 @@ def fused_projection(terms, bias, relu=True, row_scales=None):
 # ------------------------------------------------------------------------------------------
 # K5: score contraction + top-k (inference.py:427-428)
 # ------------------------------------------------------------------------------------------
-def score_topk(q: torch.Tensor, cat: torch.Tensor, k: int, id_offset: int = 0):
+def score_topk(q: torch.Tensor, cat: torch.Tensor, k: int, id_offset: int = 0, exclude=None, rows=None):
     """``torch.topk(torch.mm(q, cat.T), min(k, len))`` without materialising the scores.
-    Returns ``(values[B,k'] fp32 descending, ids[B,k'] int64)`` under (score desc, id asc)."""
+    Returns ``(values[B,k'] fp32 descending, ids[B,k'] int64)`` under (score desc, id asc).
+
+    ``exclude``: an ``ExclusionIndex``; query ``b`` then never gets a post id of exclusion row
+    ``rows[b]`` (``rows``: int64 ``[B]`` on the device, each in ``[0, exclude.num_rows)``; default: row
+    ``b``).  A query with fewer than ``k'`` admissible posts is padded at its tail with
+    ``(-inf, -1)``.  ``exclude=None`` is exactly the call without exclusions."""
     lib = _lib.load()
     if q.dim() == 1:
         q = q.unsqueeze(0)
@@ -536,15 +541,33 @@ def score_topk(q: torch.Tensor, cat: torch.Tensor, k: int, id_offset: int = 0):
     b, h = q.shape
     p = cat.size(0)
     kk = min(int(k), p)
+    if exclude is None and rows is not None:
+        raise ValueError("score_topk: rows selects exclusion rows and needs exclude")
+    if exclude is not None:
+        if rows is None:
+            if b > exclude.num_rows:
+                raise ValueError(f"score_topk: {b} queries but the exclusion index has {exclude.num_rows} rows; "
+                                 "pass rows= to map queries to rows")
+        else:
+            if rows.dtype != torch.int64 or rows.dim() != 1 or rows.numel() != b:
+                raise ValueError(f"score_topk: rows must be int64 [B={b}]")
+            rows = rows.contiguous()
     vals = torch.empty(b, kk, dtype=torch.float32, device=q.device)
     ids = torch.empty(b, kk, dtype=torch.int64, device=q.device)
     if b == 0 or kk == 0:
         return vals, ids
     ws_bytes = int(lib.trg_score_topk_workspace_bytes(b, p, h, kk))
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=q.device)
-    _lib.call("trg_score_topk", 2 * b * p * h, lib.trg_score_topk,  # "bytes" slot carries flops here
-              _lib.ptr(q), _lib.ptr(cat), b, p, h, _lib.dtype_code(q.dtype), kk, int(id_offset),
-              _lib.ptr(vals), _lib.ptr(ids), _lib.ptr(ws), ws_bytes, _lib.stream())
+    if exclude is None:
+        _lib.call("trg_score_topk", 2 * b * p * h, lib.trg_score_topk,  # "bytes" slot carries flops here
+                  _lib.ptr(q), _lib.ptr(cat), b, p, h, _lib.dtype_code(q.dtype), kk, int(id_offset),
+                  _lib.ptr(vals), _lib.ptr(ids), _lib.ptr(ws), ws_bytes, _lib.stream())
+    else:
+        _lib.call("trg_score_topk_excluding", 2 * b * p * h, lib.trg_score_topk_excluding,
+                  _lib.ptr(q), _lib.ptr(cat), b, p, h, _lib.dtype_code(q.dtype), kk, int(id_offset),
+                  # an index without any id: every row is empty and no id is read, but the pointer must be valid
+                  _lib.ptr(exclude.rowptr), _lib.ptr(exclude.ids if exclude.nnz else exclude.rowptr), _lib.ptr(rows),
+                  _lib.ptr(vals), _lib.ptr(ids), _lib.ptr(ws), ws_bytes, _lib.stream())
     return vals, ids
 
 

@@ -154,7 +154,8 @@ def train_step(model, optimizer, x_dict, edge_index_dict, train_edge_index, inte
 
 
 @torch.no_grad()
-def recommend(user_emb, known_post_emb, k=10, id_offset=0):
+def recommend(user_emb, known_post_emb, k=10, id_offset=0, exclude=None, rows=None):
     """``scores = torch.mm(user_emb, known_post_emb.T); torch.topk(scores, min(K, len(scores)))``
-    (inference.py:427-428) for one user row or a batch.  Returns ``(top scores, top post ids)``."""
-    return score_topk(user_emb, known_post_emb, k, id_offset)
+    (inference.py:427-428) for one user row or a batch.  Returns ``(top scores, top post ids)``.
+    ``exclude`` / ``rows``: drop each user's history (an ``ExclusionIndex``), see ``score_topk``."""
+    return score_topk(user_emb, known_post_emb, k, id_offset, exclude=exclude, rows=rows)
