@@ -14,7 +14,8 @@ every collective of the step is in flight while an independent kernel runs:
 
 Collectives are ``torch.distributed`` async ops (NCCL runs them on its own stream over NVLink /
 NVSwitch); ``wait()`` only orders the consuming kernel after them.  ReLU backward and gradient
-accumulation ride in kernel epilogues as in ``fused_step``.  ``prims`` supplies the compute
+accumulation ride in kernel epilogues and the layer's GEMMs come from the model, as in ``fused_step``;
+the graphed step is a ``train.GraphedStep``.  ``prims`` supplies the compute
 primitives: the CUDA kernels in the product (``CUDA_STEP_PRIMS``), oracle ops in the CPU (gloo)
 tests of this host logic (``tests/oracle_ops.OracleStepPrims``).
 """
@@ -23,9 +24,12 @@ from __future__ import annotations
 import torch
 import torch.distributed as dist
 
+from . import _lib
 from .dist import PaddedPairs, ShardedGraph, allreduce_grads
+from .fused_step import _agg, _layers, model_eligible
 from .graph import PushRelation
-from .nn import REL_DIRECT, REL_ENGAGE, REL_SOCIAL, StackedWeightedRGCN, WeightedRGCN
+from .nn import REL_DIRECT, REL_ENGAGE, REL_SOCIAL
+from .train import GraphedStep
 
 
 # ------------------------------------------------------------------------------------------
@@ -143,10 +147,7 @@ def comm_for(model, shard: ShardedGraph):
 class CudaStepPrims:
     """The sm_100a kernels, by the names the step below uses."""
 
-    @staticmethod
-    def agg_mean(rel, x_src):
-        from .fused_step import _agg
-        return _agg(rel, x_src)
+    agg_mean = staticmethod(_agg)                       # (rel, x_src)
 
     @staticmethod
     def gather_sum(rel, which, x, out=None, accumulate=False, relu_of=None, out_dtype=None):
@@ -209,23 +210,18 @@ def transport_dtype(dtype):
     return torch.float32 if dtype == torch.bfloat16 else None
 
 
-def _accum(param, grad):
-    grad = grad.to(param.dtype)
-    if param.grad is None:
-        param.grad = grad
-    else:
-        param.grad.add_(grad)
-
-
 def eligible(model, shard: ShardedGraph) -> bool:
-    if type(model) not in (WeightedRGCN, StackedWeightedRGCN) or shard.world < 2 or not torch.is_grad_enabled():
-        return False
-    if not isinstance(shard.rels[REL_DIRECT], PushRelation):
-        return False
-    layers = list(model.layers) if type(model) is StackedWeightedRGCN else [model]
-    if any(conv.lin_l.bias is None for l in layers for conv in (l.msg_direct, l.msg_social, l.post_update)):
-        return False
-    return all(p.requires_grad for p in model.parameters())
+    """``fused_step.model_eligible`` on a shard of two or more ranks with the post -> user relation pushed."""
+    return shard.world >= 2 and isinstance(shard.rels[REL_DIRECT], PushRelation) and model_eligible(model)
+
+
+def _host_slice_gather(shard: ShardedGraph, host: torch.Tensor):
+    """The shard's ``HostSliceGather`` for host arrays the size of ``host``, cached as ``shard._neg_gather``."""
+    hg = getattr(shard, "_neg_gather", None)
+    if hg is None or hg.n != host.numel():
+        from .peer import HostSliceGather
+        hg = shard._neg_gather = HostSliceGather(host.numel(), host.dtype, shard.x_local["user"].device)
+    return hg
 
 
 @torch.no_grad()
@@ -236,7 +232,9 @@ def loss_and_grads_sharded(model, shard: ShardedGraph, neg_p_local, prims=CUDA_S
     both).  Negatives: ``neg_p_local`` = ``shard.local_negatives(neg_p)`` (or a ``PaddedPairs``), or
     ``neg_p_global`` = the step's full ``neg_p`` -- this rank's share is then selected here, on the device
     and without a host sync, while the final user rows are being all-gathered."""
-    layers = list(model.layers) if type(model) is StackedWeightedRGCN else [model]
+    layers = _layers(model)
+    if layers is None:
+        raise _lib.TrgError("loss_and_grads_sharded: model must be WeightedRGCN or StackedWeightedRGCN")
     prel_d, rel_s, rel_e = shard.rels[REL_DIRECT], shard.rels[REL_SOCIAL], shard.rels[REL_ENGAGE]
     rel_d = prel_d.rel                                  # rows ("fwd") = all users, sources = local posts
     hu, hp = shard.x_local["user"], shard.x_local["post"]
@@ -250,11 +248,7 @@ def loss_and_grads_sharded(model, shard: ShardedGraph, neg_p_local, prims=CUDA_S
     # ---- forward ----
     saved = []
     for i, layer in enumerate(layers):
-        d, s, p = layer.msg_direct, layer.msg_social, layer.post_update
-        for conv, (xs, xd) in ((d, (hp, hu)), (s, (hu, hu)), (p, (hu, hp))):
-            conv.lin_l.materialize(xs.size(-1))
-            conv.lin_r.materialize(xd.size(-1))
-        wd, ws = float(layer.w_direct), float(layer.w_social)
+        layer.materialize(hu.size(-1), hp.size(-1))
         ag = None if i == 0 else comm.all_gather_rows_async(hu)
         part = prims.gather_sum(rel_d, "fwd", hp, out=comm.partial(n_u_pad, hp.size(1), pdt),
                                 out_dtype=xfer)                          # [U_pad, F] partial sums  || all-gather
@@ -264,13 +258,12 @@ def loss_and_grads_sharded(model, shard: ShardedGraph, neg_p_local, prims=CUDA_S
         mean_s = prims.agg_mean(rel_s, user_full)                        # || reduce-scatter
         mean_e = prims.agg_mean(rel_e, user_full)
         del user_full
-        hp_n = prims.proj_fwd([(mean_e, p.lin_l.weight, 1.0), (hp, p.lin_r.weight, 1.0)], p.lin_l.bias, True)
+        pg = layer.post_gemm()
+        hp_n = prims.proj_fwd(pg.terms(mean_e, hp), pg.bias, True)
         mean_d = rs.wait()
-        w_root = wd * d.lin_r.weight + ws * s.lin_r.weight
-        b_user = wd * d.lin_l.bias + ws * s.lin_l.bias
-        hu_n = prims.proj_fwd([(mean_d, d.lin_l.weight, wd), (mean_s, s.lin_l.weight, ws), (hu, w_root, 1.0)],
-                              b_user, True)
-        saved.append((hu, hp, mean_d, mean_s, mean_e, w_root))
+        ug = layer.user_gemm()
+        hu_n = prims.proj_fwd(ug.terms(mean_d, mean_s, hu), ug.bias, True)
+        saved.append((hu, hp, mean_d, mean_s, mean_e, ug, pg))
         hu, hp = hu_n, hp_n
 
     # ---- loss: every <u, p> term is evaluated by the owner of the post (dist.ShardedGraph) ----
@@ -302,36 +295,24 @@ def loss_and_grads_sharded(model, shard: ShardedGraph, neg_p_local, prims=CUDA_S
 
     # ---- backward ----
     for li in range(len(layers) - 1, -1, -1):
-        layer = layers[li]
-        d, s, p = layer.msg_direct, layer.msg_social, layer.post_update
-        wd, ws = float(layer.w_direct), float(layer.w_social)
-        hu_in, hp_in, mean_d, mean_s, mean_e, w_root = saved.pop()
+        hu_in, hp_in, mean_d, mean_s, mean_e, ug, pg = saved.pop()
         # post side first: it does not depend on the user-gradient reduce-scatter still in flight
-        (dw_p, dw_pr), db_p = prims.proj_bwd_weight(dz_p, [(mean_e, 1.0), (hp_in, 1.0)], True)
+        dw_p, db_p = prims.proj_bwd_weight(dz_p, pg.dw_terms(mean_e, hp_in), True)
         g_uf = g_hp = None
         if li > 0:
-            g_me, g_hp = prims.proj_bwd_input(dz_p, [(p.lin_l.weight, 1.0, rel_e.inv_deg), (p.lin_r.weight, 1.0, None)])
+            g_me, g_hp = prims.proj_bwd_input(dz_p, pg.dx_terms(rel_e.inv_deg, None))
             g_uf = prims.gather_sum(rel_e, "bwd", g_me, out=comm.partial(n_u_pad, g_me.size(1), pdt),
                                     out_dtype=xfer)                      # d user_full partials (engages^T)
             del g_me
         del dz_p, mean_e
         dz_u = pend_u.wait()                                  # reduced (+ local term), ReLU backward applied
         del pend_u
-        (dw_d, dw_s, dw_root), db_u = prims.proj_bwd_weight(dz_u, [(mean_d, wd), (mean_s, ws), (hu_in, 1.0)], True)
+        dw_u, db_u = prims.proj_bwd_weight(dz_u, ug.dw_terms(mean_d, mean_s, hu_in), True)
         del mean_d, mean_s
-        _accum(d.lin_l.weight, dw_d)
-        _accum(s.lin_l.weight, dw_s)
-        _accum(d.lin_r.weight, wd * dw_root)
-        _accum(s.lin_r.weight, ws * dw_root)
-        _accum(d.lin_l.bias, wd * db_u)
-        _accum(s.lin_l.bias, ws * db_u)
-        _accum(p.lin_l.weight, dw_p)
-        _accum(p.lin_r.weight, dw_pr)
-        _accum(p.lin_l.bias, db_p)
+        layers[li].accumulate_grads(dw_u, db_u, dw_p, db_p)
         if li == 0:
             break
-        g_md, g_ms, g_hu = prims.proj_bwd_input(
-            dz_u, [(d.lin_l.weight, wd, prel_d.inv_deg), (s.lin_l.weight, ws, rel_s.inv_deg), (w_root, 1.0, None)])
+        g_md, g_ms, g_hu = prims.proj_bwd_input(dz_u, ug.dx_terms(prel_d.inv_deg, rel_s.inv_deg, None))
         del dz_u
         ag = comm.all_gather_rows_async(g_md)                         # every post owner needs d mean_direct
         g_uf = prims.gather_sum(rel_s, "bwd", g_ms, out=g_uf, accumulate=True)      # || all-gather
@@ -343,35 +324,22 @@ def loss_and_grads_sharded(model, shard: ShardedGraph, neg_p_local, prims=CUDA_S
     return loss_local
 
 
-class GraphedShardedStep:
+class GraphedShardedStep(GraphedStep):
     """The sharded step -- forward, loss, backward, every collective, the gradient all-reduce -- captured ONCE
-    into a CUDA graph and replayed per step (``train_step_sharded_fused(..., cuda_graph=True)``).
+    into a CUDA graph and replayed per step (``train_step_sharded_fused(..., cuda_graph=True)``; the capture and
+    replay are :class:`train.GraphedStep`'s).
 
     At 8 GPUs one step is ~9 ms of GPU work behind ~85 kernel launches, ~60 copy-engine transfers and ~120
     stream/event operations: enqueueing them from Python takes as long as executing them (9 - 11 ms measured),
-    so the eager step is host-bound.  The replay is one launch.  What stays outside the graph: the upload of
-    this step's negatives into the graph's static input (``HostSliceGather`` for host arrays), the optimiser's
-    own ``step()`` (the caller's ``torch.optim`` object, untouched) and the loss read-back.
-
-    Capture happens on the first call, after two eager steps' worth of warm-up with that call's negatives
-    (structures and lazy weights materialise there; the optimiser is NOT stepped during warm-up).  The
-    parameters' ``.grad`` tensors live in the graph's memory pool and are rewritten by every replay, so
-    ``optimizer.zero_grad()`` is not needed (and must not set them to None) between graphed steps."""
+    so the eager step is host-bound.  The replay is one launch.  Host negatives are uploaded with the shard's
+    ``HostSliceGather`` when the ranks share peer memory."""
 
     def __init__(self, model, optimizer, shard: ShardedGraph, neg_capacity=None):
         if not eligible(model, shard) or not shard.x_local["user"].is_cuda:
             raise ValueError("GraphedShardedStep needs a CUDA shard and a model the tape-free sharded step accepts")
-        self.model, self.optimizer, self.shard, self.neg_capacity = model, optimizer, shard, neg_capacity
+        super().__init__(model, optimizer, shard.n_pos_global, shard.x_local["user"].device)
+        self.shard, self.neg_capacity = shard, neg_capacity
         self.comm = comm_for(model, shard)
-        dev = shard.x_local["user"].device
-        self.neg = torch.empty(shard.n_pos_global, dtype=torch.int64, device=dev)
-        # "this step's negatives are in self.neg": an EXTERNAL event -- inside the graph it is an event-wait
-        # node placed right before the negatives are first read (the loss), so the upload of a step's host
-        # negatives overlaps the replayed forward pass exactly as in the eager step
-        self.neg_ready = torch.cuda.Event(external=True)
-        self.graph = None
-        self.loss = None
-        self.launches_per_replay = 0
 
     def _body(self):
         loss = loss_and_grads_sharded(self.model, self.shard, None, CUDA_STEP_PRIMS, neg_ready=self.neg_ready,
@@ -381,60 +349,21 @@ class GraphedShardedStep:
         lw.wait()
         return loss
 
-    def _capture(self):
-        from . import _lib
-        if _lib.PROF.enabled:
-            raise _lib.TrgError("GraphedShardedStep: per-call event timing (PROF) cannot run inside a graph capture")
-        cur = torch.cuda.current_stream()
-        side = torch.cuda.Stream(self.neg.device)
-        side.wait_stream(cur)
-        with torch.cuda.stream(side):
-            for _ in range(2):                       # warm-up: structures, lazy weights, allocator
-                self.optimizer.zero_grad(set_to_none=True)
-                self._body()
-        cur.wait_stream(side)
-        torch.cuda.synchronize()
-        dist.barrier()
-        self.optimizer.zero_grad(set_to_none=True)
-        if isinstance(self.comm, PeerMemoryComm):
-            self.comm.pc._last_barrier = None        # an event recorded outside the capture cannot be waited inside
-        g = torch.cuda.CUDAGraph()
-        n0 = _lib.launch_count()
-        with torch.cuda.graph(g, capture_error_mode="thread_local"):
-            self.loss = self._body()
-        self.launches_per_replay = _lib.launch_count() - n0      # kernels of this library inside one replay
-        self.params = [p for p in self.model.parameters() if p.grad is not None]
-        self.grads = [p.grad for p in self.params]               # static: rewritten by every replay
-        self.graph = g
+    def _draw_negatives(self):
+        return self.shard.draw_negatives()
 
-    def close(self):
-        """Drop the captured graph (and with it the NCCL work it holds): a process group must not be destroyed
-        while a graph that captured its collectives is alive."""
-        self.graph = None
-        self.loss = None
-        self.params, self.grads = [], []
-
-    def __call__(self, neg_p_global, return_tensor=False):
-        shard = self.shard
-        self.model.train()
-        if neg_p_global is None:
-            neg_p_global = shard.draw_negatives()
+    def _upload(self, neg_p_global):
         if not neg_p_global.is_cuda and isinstance(self.comm, PeerMemoryComm):
-            hg = getattr(shard, "_neg_gather", None)
-            if hg is None or hg.n != neg_p_global.numel():
-                from .peer import HostSliceGather
-                hg = shard._neg_gather = HostSliceGather(neg_p_global.numel(), neg_p_global.dtype, self.neg.device)
+            hg = _host_slice_gather(self.shard, neg_p_global)
             hg.gather_async(neg_p_global, out=self.neg, event=self.neg_ready)     # side stream: overlaps the forward
         else:
             self.neg.copy_(neg_p_global, non_blocking=True)
             self.neg_ready.record()
-        if self.graph is None:
-            self._capture()
-        self.graph.replay()
-        for p, g in zip(self.params, self.grads):                # (an eager step in between may have re-pointed them)
-            p.grad = g
-        self.optimizer.step()
-        return self.loss if return_tensor else self.loss.item()
+
+    def _before_capture(self):
+        dist.barrier()
+        if isinstance(self.comm, PeerMemoryComm):
+            self.comm.pc._last_barrier = None        # an event recorded outside the capture cannot be waited inside
 
 
 def train_step_sharded_fused(model, optimizer, shard: ShardedGraph, neg_p_global=None, neg_p_local=None,
@@ -464,12 +393,7 @@ def train_step_sharded_fused(model, optimizer, shard: ShardedGraph, neg_p_global
         if not neg_p_global.is_cuda and is_cuda:
             if prims is CUDA_STEP_PRIMS and isinstance(comm_for(model, shard), PeerMemoryComm):
                 # every rank holds the same host array: upload 1/G of it, pull the rest over NVLink
-                hg = getattr(shard, "_neg_gather", None)
-                if hg is None or hg.n != neg_p_global.numel():
-                    from .peer import HostSliceGather
-                    hg = shard._neg_gather = HostSliceGather(neg_p_global.numel(), neg_p_global.dtype,
-                                                             shard.x_local["user"].device)
-                neg_p_global, neg_ready = hg.gather_async(neg_p_global)
+                neg_p_global, neg_ready = _host_slice_gather(shard, neg_p_global).gather_async(neg_p_global)
             else:
                 from .train import stage_negatives
                 neg_p_global, neg_ready = stage_negatives(neg_p_global, shard.x_local["user"].device)

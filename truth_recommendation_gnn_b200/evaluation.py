@@ -58,15 +58,11 @@ def embed_cold_users(model, x_user):
     """Embeddings of users with no edges (inference.py:397-424): every SAGEConv sees E = 0, so
     ``user_emb = relu(w_direct*(b_d + x W_r,d^T) + w_social*(b_s + x W_r,s^T))`` -- one fused K3
     launch for the whole batch instead of a 1-node ``HeteroData`` + forward per user."""
-    d, s = model.msg_direct, model.msg_social
-    d.lin_r.materialize(x_user.size(-1))
-    s.lin_r.materialize(x_user.size(-1))
-    wd, ws = float(model.w_direct), float(model.w_social)
-    w_root = (wd * d.lin_r.weight + ws * s.lin_r.weight).contiguous()
-    bias = None
-    if d.lin_l.bias is not None:
-        bias = wd * d.lin_l.bias + ws * s.lin_l.bias
-    return sage_proj_fwd([(x_user.contiguous(), w_root, 1.0)], bias, True)
+    model.msg_direct.lin_r.materialize(x_user.size(-1))
+    model.msg_social.lin_r.materialize(x_user.size(-1))
+    ug = model.user_gemm()
+    # both means are zero: only the root term, the user GEMM's last operand, remains
+    return sage_proj_fwd([(x_user.contiguous(), ug.weights[-1], ug.alphas[-1])], ug.bias, True)
 
 
 @torch.no_grad()

@@ -12,6 +12,9 @@ between them disappear into kernel epilogues:
   aggregation + root term; post rows: rev_engages aggregation + root term) -> ``accumulate`` into the
   root-term gradient written by the projection backward.
 
+Each layer's two GEMMs take their operands from the model (``WeightedRGCN.user_gemm`` / ``post_gemm``) and
+hand their gradients back through ``accumulate_grads``, as the autograd and sharded (``dist_fused``) steps do.
+
 At config 2 this removes ~20 GB of element-wise HBM traffic per step.  The autograd path
 (``functional.py`` Functions) stays the general one; ``train_step`` takes this path when the model,
 inputs and parameters qualify (``eligible``) and both are checked against each other and against the
@@ -29,6 +32,7 @@ from .nn import REL_DIRECT, REL_ENGAGE, REL_SOCIAL, StackedWeightedRGCN, Weighte
 
 
 def _layers(model):
+    """The layers of the reference model classes (not subclasses with a changed forward), else None."""
     if type(model) is StackedWeightedRGCN:
         return list(model.layers)
     if type(model) is WeightedRGCN:
@@ -36,29 +40,24 @@ def _layers(model):
     return None
 
 
-def eligible(model, x_dict) -> bool:
-    """True when the tape-free path computes the same thing as autograd would: the reference model
-    classes (not subclasses with a changed forward), leaf inputs that need no gradient, CUDA."""
+def model_eligible(model) -> bool:
+    """The model-side conditions of the tape-free steps (this one and ``dist_fused``): a reference model class,
+    every conv with its bias, every parameter requiring a gradient, grad mode enabled."""
     layers = _layers(model)
     if layers is None or not torch.is_grad_enabled():
         return False
-    xu, xp = x_dict["user"], x_dict["post"]
-    if not (xu.is_cuda and xp.is_cuda) or xu.requires_grad or xp.requires_grad or xu.dtype != xp.dtype:
+    if any(conv.lin_l.bias is None for l in layers for conv in (l.msg_direct, l.msg_social, l.post_update)):
         return False
-    for layer in layers:
-        for conv in (layer.msg_direct, layer.msg_social, layer.post_update):
-            if conv.lin_l.bias is None:
-                return False
     return all(p.requires_grad for p in model.parameters())
 
 
-def _accum(param, grad):
-    """What ``loss.backward()`` does with a leaf gradient."""
-    grad = grad.to(param.dtype)
-    if param.grad is None:
-        param.grad = grad
-    else:
-        param.grad.add_(grad)
+def eligible(model, x_dict) -> bool:
+    """True when the tape-free path computes the same thing as autograd would: ``model_eligible``, and leaf
+    CUDA inputs of one dtype that need no gradient."""
+    if not model_eligible(model):
+        return False
+    xu, xp = x_dict["user"], x_dict["post"]
+    return xu.is_cuda and xp.is_cuda and not xu.requires_grad and not xp.requires_grad and xu.dtype == xp.dtype
 
 
 def _agg(rel, x):
@@ -86,18 +85,12 @@ def loss_and_grads(model, x_dict, edge_index_dict, train_edge_index, interaction
     # ---- forward (train_gnn.py:166-200 per layer) ----
     saved = []
     for layer in layers:
-        d, s, p = layer.msg_direct, layer.msg_social, layer.post_update
-        for conv, (xs, xd) in ((d, (hp, hu)), (s, (hu, hu)), (p, (hu, hp))):
-            conv.lin_l.materialize(xs.size(-1))
-            conv.lin_r.materialize(xd.size(-1))
-        wd, ws = float(layer.w_direct), float(layer.w_social)
+        layer.materialize(hu.size(-1), hp.size(-1))
         mean_d, mean_s, mean_e = _agg(rel_d, hp), _agg(rel_s, hu), _agg(rel_e, hu)
-        w_root = wd * d.lin_r.weight + ws * s.lin_r.weight
-        b_user = wd * d.lin_l.bias + ws * s.lin_l.bias
-        hu_n = sage_proj_fwd([(mean_d, d.lin_l.weight, wd), (mean_s, s.lin_l.weight, ws), (hu, w_root, 1.0)],
-                             b_user, True)
-        hp_n = sage_proj_fwd([(mean_e, p.lin_l.weight, 1.0), (hp, p.lin_r.weight, 1.0)], p.lin_l.bias, True)
-        saved.append((hu, hp, mean_d, mean_s, mean_e, w_root))
+        ug, pg = layer.user_gemm(), layer.post_gemm()
+        hu_n = sage_proj_fwd(ug.terms(mean_d, mean_s, hu), ug.bias, True)
+        hp_n = sage_proj_fwd(pg.terms(mean_e, hp), pg.bias, True)
+        saved.append((hu, hp, mean_d, mean_s, mean_e, ug, pg))
         hu, hp = hu_n, hp_n
 
     # ---- loss (train_gnn.py:259-281) + its backward onto the last layer's pre-activations ----
@@ -129,29 +122,17 @@ def loss_and_grads(model, x_dict, edge_index_dict, train_edge_index, interaction
 
     # ---- backward through the layers (train_gnn.py:283) ----
     for li in range(len(layers) - 1, -1, -1):
-        layer = layers[li]
-        d, s, p = layer.msg_direct, layer.msg_social, layer.post_update
-        wd, ws = float(layer.w_direct), float(layer.w_social)
-        hu_in, hp_in, mean_d, mean_s, mean_e, w_root = saved.pop()
-        (dw_d, dw_s, dw_root), db_u = sage_proj_bwd_weight(dz_u, [(mean_d, wd), (mean_s, ws), (hu_in, 1.0)], True)
-        (dw_p, dw_pr), db_p = sage_proj_bwd_weight(dz_p, [(mean_e, 1.0), (hp_in, 1.0)], True)
+        hu_in, hp_in, mean_d, mean_s, mean_e, ug, pg = saved.pop()
+        dw_u, db_u = sage_proj_bwd_weight(dz_u, ug.dw_terms(mean_d, mean_s, hu_in), True)
+        dw_p, db_p = sage_proj_bwd_weight(dz_p, pg.dw_terms(mean_e, hp_in), True)
         del mean_d, mean_s, mean_e
-        _accum(d.lin_l.weight, dw_d)
-        _accum(s.lin_l.weight, dw_s)
-        _accum(d.lin_r.weight, wd * dw_root)
-        _accum(s.lin_r.weight, ws * dw_root)
-        _accum(d.lin_l.bias, wd * db_u)
-        _accum(s.lin_l.bias, ws * db_u)
-        _accum(p.lin_l.weight, dw_p)
-        _accum(p.lin_r.weight, dw_pr)
-        _accum(p.lin_l.bias, db_p)
+        layers[li].accumulate_grads(dw_u, db_u, dw_p, db_p)
         if li == 0:
             break
         # gradients w.r.t. this layer's inputs = the previous layer's outputs; the mean terms come out
         # pre-scaled by 1/deg, so the transposed aggregations below are plain gather-sums
-        g_md, g_ms, g_hu = sage_proj_bwd_input(
-            dz_u, [(d.lin_l.weight, wd, rel_d.inv_deg), (s.lin_l.weight, ws, rel_s.inv_deg), (w_root, 1.0, None)])
-        g_me, g_hp = sage_proj_bwd_input(dz_p, [(p.lin_l.weight, 1.0, rel_e.inv_deg), (p.lin_r.weight, 1.0, None)])
+        g_md, g_ms, g_hu = sage_proj_bwd_input(dz_u, ug.dx_terms(rel_d.inv_deg, rel_s.inv_deg, None))
+        g_me, g_hp = sage_proj_bwd_input(dz_p, pg.dx_terms(rel_e.inv_deg, None))
         del dz_u, dz_p
         sage_agg_bwd(rel_s.bwd, None, g_ms, out=g_hu, accumulate=True)
         sage_agg_bwd(rel_e.bwd, None, g_me, out=g_hu, accumulate=True, relu_of=hu_in)

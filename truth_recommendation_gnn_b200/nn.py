@@ -13,6 +13,7 @@ ReLU fused.
 from __future__ import annotations
 
 import math
+from typing import NamedTuple
 
 import torch
 import torch.nn.functional as F
@@ -132,9 +133,43 @@ class SAGEConv(torch.nn.Module):
         return f"SAGEConv({self.in_channels}, {self.out_channels}, aggr=mean)"
 
 
+class FusedGemm(NamedTuple):
+    """One fused K3 projection, ``relu(sum_t alphas[t] * A_t @ weights[t]^T + bias)`` with one operand A_t per
+    weight, and the term lists of its forward (``terms``) and backward (``dw_terms``, ``dx_terms``) kernels."""
+    weights: tuple
+    alphas: tuple
+    bias: torch.Tensor | None
+
+    def terms(self, *operands):             # [(A, W, alpha)]: sage_proj_fwd, fused_projection
+        return list(zip(operands, self.weights, self.alphas, strict=True))
+
+    def dw_terms(self, *operands):          # [(A, alpha)]: sage_proj_bwd_weight
+        return list(zip(operands, self.alphas, strict=True))
+
+    def dx_terms(self, *row_scales):        # [(W, alpha, row scale)]: sage_proj_bwd_input
+        return list(zip(self.weights, self.alphas, row_scales, strict=True))
+
+
+def _accum(param, grad):
+    """What ``loss.backward()`` does with a leaf gradient."""
+    grad = grad.to(param.dtype)
+    if param.grad is None:
+        param.grad = grad
+    else:
+        param.grad.add_(grad)
+
+
 class WeightedRGCN(torch.nn.Module):
     """The reference model, train_gnn.py:147-200 (dup inference.py:119-169): same attribute names,
-    same fixed python-float relation weights, same ``forward(x_dict, edge_index_dict)``."""
+    same fixed python-float relation weights, same ``forward(x_dict, edge_index_dict)``.
+
+    Every path that runs the layer (autograd, tape-free, sharded, cold-start) computes it as two GEMMs
+    whose operands come from ``user_gemm`` / ``post_gemm`` (wd, ws = ``w_direct``, ``w_social``)::
+
+        user = relu([mean_d | mean_s | x_u] @ [wd W_l,d | ws W_l,s | wd W_r,d + ws W_r,s]^T + wd b_d + ws b_s)
+        post = relu([mean_e | x_p] @ [W_l,e | W_r,p]^T + b_e)
+
+    and ``accumulate_grads`` maps the GEMMs' gradients back onto the nine parameters."""
 
     def __init__(self, hidden_dim=64, in_channels=(-1, -1)):
         super().__init__()
@@ -143,6 +178,44 @@ class WeightedRGCN(torch.nn.Module):
         self.post_update = SAGEConv(in_channels, hidden_dim)  # post <- user (engagement)
         self.w_direct = 1.0
         self.w_social = 0.75
+
+    def materialize(self, user_feat: int, post_feat: int):
+        """Resolve the convs' lazy in-channels from the user and post feature widths."""
+        widths = ((post_feat, user_feat), (user_feat, user_feat), (user_feat, post_feat))
+        for conv, (f_src, f_dst) in zip((self.msg_direct, self.msg_social, self.post_update), widths):
+            conv.lin_l.materialize(f_src)
+            conv.lin_r.materialize(f_dst)
+
+    def user_gemm(self) -> FusedGemm:
+        """Operands ``[mean_d | mean_s | x_u]``; the root weight and bias are combined anew by every call."""
+        d, s = self.msg_direct, self.msg_social
+        wd, ws = float(self.w_direct), float(self.w_social)
+        w_root = wd * d.lin_r.weight + ws * s.lin_r.weight
+        b_user = None
+        if d.lin_l.bias is not None:
+            b_user = wd * d.lin_l.bias + ws * s.lin_l.bias
+        return FusedGemm((d.lin_l.weight, s.lin_l.weight, w_root), (wd, ws, 1.0), b_user)
+
+    def post_gemm(self) -> FusedGemm:
+        """Operands ``[mean_e | x_p]``."""
+        p = self.post_update
+        return FusedGemm((p.lin_l.weight, p.lin_r.weight), (1.0, 1.0), p.lin_l.bias)
+
+    def accumulate_grads(self, dw_user, db_user, dw_post, db_post):
+        """Add both GEMMs' gradients (one dW per operand, db) to the nine parameters as ``loss.backward()`` does."""
+        d, s, p = self.msg_direct, self.msg_social, self.post_update
+        wd, ws = float(self.w_direct), float(self.w_social)
+        dw_d, dw_s, dw_root = dw_user
+        dw_p, dw_pr = dw_post
+        _accum(d.lin_l.weight, dw_d)
+        _accum(s.lin_l.weight, dw_s)
+        _accum(d.lin_r.weight, wd * dw_root)
+        _accum(s.lin_r.weight, ws * dw_root)
+        _accum(d.lin_l.bias, wd * db_user)
+        _accum(s.lin_l.bias, ws * db_user)
+        _accum(p.lin_l.weight, dw_p)
+        _accum(p.lin_r.weight, dw_pr)
+        _accum(p.lin_l.bias, db_post)
 
     def forward(self, x_dict, edge_index_dict):
         """Same result as train_gnn.py:166-200, computed as three K1 aggregations and two fused
@@ -165,25 +238,15 @@ class WeightedRGCN(torch.nn.Module):
         ``src_dict is dst_dict``."""
         user_src, post_src = src_dict["user"], src_dict["post"]
         user_x, post_x = dst_dict["user"], dst_dict["post"]
-        d, s, p = self.msg_direct, self.msg_social, self.post_update
-        for conv, (xs, xd) in ((d, (post_src, user_x)), (s, (user_src, user_x)), (p, (user_src, post_x))):
-            conv.lin_l.materialize(xs.size(-1))
-            conv.lin_r.materialize(xd.size(-1))
+        self.materialize(user_x.size(-1), post_x.size(-1))
         rel_d, rel_s, rel_e = rels[REL_DIRECT], rels[REL_SOCIAL], rels[REL_ENGAGE]
         mean_d = ops.aggregate(post_src, rel_d)
         mean_s = ops.aggregate(user_src, rel_s)
         mean_e = ops.aggregate(user_src, rel_e)
-        wd, ws = float(self.w_direct), float(self.w_social)
-        w_root = wd * d.lin_r.weight + ws * s.lin_r.weight
-        b_user = None
-        if d.lin_l.bias is not None:
-            b_user = wd * d.lin_l.bias + ws * s.lin_l.bias
-        user_out = ops.project(
-            [(mean_d, d.lin_l.weight, wd), (mean_s, s.lin_l.weight, ws), (user_x, w_root, 1.0)],
-            b_user, True, (rel_d, rel_s, None))
-        post_out = ops.project(
-            [(mean_e, p.lin_l.weight, 1.0), (post_x, p.lin_r.weight, 1.0)],
-            p.lin_l.bias, True, (rel_e, None))
+        ug = self.user_gemm()
+        user_out = ops.project(ug.terms(mean_d, mean_s, user_x), ug.bias, True, (rel_d, rel_s, None))
+        pg = self.post_gemm()
+        post_out = ops.project(pg.terms(mean_e, post_x), pg.bias, True, (rel_e, None))
         return {"user": user_out, "post": post_out}
 
 

@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import torch
 
-from . import fused_step
+from . import _lib, fused_step
 from .functional import link_bce_loss, score_topk
 
 
@@ -34,29 +34,85 @@ def stage_negatives(neg_p, device):
     return dev_t, ev
 
 
-class GraphedTrainStep:
-    """``train_step`` replayed from a CUDA graph: forward + loss + backward (the tape-free step) are captured on
-    the first call and launched as one graph per step afterwards.  At the reference's own scale (BASELINE config
-    1: 10k users / 50k posts / 500k edges) a step is ~32 launches of a few microseconds each and the eager step
-    is bound by Python's launch path (~1 ms); the replay is one launch.  At config 2 the step is GPU-bound and
-    the graph changes nothing.  Outside the graph: the upload of the step's negatives into the graph's static
-    input (an ``external`` event orders the loss after it, so a host array still uploads during the forward),
-    the caller's own ``optimizer.step()`` and the loss read-back.  The static inputs (features, edge lists) are
-    the tensors of the first call: a different graph object needs a new ``GraphedTrainStep``."""
+class GraphedStep:
+    """A tape-free train step (subclasses supply ``_body``, ``_draw_negatives``, ``_upload``) captured into a
+    CUDA graph on the first call, after two warm-up passes with that call's negatives (structures and lazy
+    weights materialise there; the optimiser is NOT stepped), and replayed as one launch per step.  Outside the
+    graph: ``_upload`` of the step's negatives into the static input ``neg``, ending with ``neg_ready``, an
+    ``external`` event whose wait node sits right before the loss, so a host array still uploads during the
+    replayed forward; the caller's ``optimizer.step()``; the loss read-back.  The ``.grad`` tensors live in the
+    graph's pool and are rewritten by every replay: ``optimizer.zero_grad()`` must not set them to None."""
+
+    def __init__(self, model, optimizer, n_neg, device):
+        self.model, self.optimizer = model, optimizer
+        self.neg = torch.empty(n_neg, dtype=torch.int64, device=device)
+        self.neg_ready = torch.cuda.Event(external=True)
+        self.graph = self.loss = None
+        self.params, self.grads, self.launches_per_replay = [], [], 0
+
+    def _before_capture(self):
+        pass
+
+    def _capture(self):
+        if _lib.PROF.enabled:
+            raise _lib.TrgError(f"{type(self).__name__}: per-call event timing (PROF) cannot run in a graph capture")
+        cur = torch.cuda.current_stream()
+        warm = torch.cuda.Stream(self.neg.device)
+        warm.wait_stream(cur)
+        with torch.cuda.stream(warm):
+            for _ in range(2):            # structures (CSRs), lazy weights, allocator; the optimiser is not stepped
+                self.optimizer.zero_grad(set_to_none=True)
+                self._body()
+        cur.wait_stream(warm)
+        torch.cuda.synchronize()
+        self._before_capture()
+        self.optimizer.zero_grad(set_to_none=True)
+        g = torch.cuda.CUDAGraph()
+        n0 = _lib.launch_count()
+        with torch.cuda.graph(g, capture_error_mode="thread_local"):
+            self.loss = self._body()
+        self.launches_per_replay = _lib.launch_count() - n0      # kernels of this library inside one replay
+        self.params = [p for p in self.model.parameters() if p.grad is not None]
+        self.grads = [p.grad for p in self.params]               # static: rewritten by every replay
+        self.graph = g
+
+    def close(self):
+        """Drop the captured graph (and with it any collective work it holds): a process group must not be
+        destroyed while a graph that captured its collectives is alive."""
+        self.graph = None
+        self.loss = None
+        self.params, self.grads = [], []
+
+    def __call__(self, neg_p=None, return_tensor=False):
+        self.model.train()
+        if neg_p is None:
+            neg_p = self._draw_negatives()
+        self._upload(neg_p)
+        if self.graph is None:
+            self._capture()
+        self.graph.replay()
+        for p, g in zip(self.params, self.grads):                # (an eager step in between may have re-pointed them)
+            p.grad = g
+        self.optimizer.step()
+        return self.loss if return_tensor else self.loss.item()
+
+
+class GraphedTrainStep(GraphedStep):
+    """``train_step`` replayed from a CUDA graph (:class:`GraphedStep`).  At the reference's own scale (BASELINE
+    config 1: 10k users / 50k posts / 500k edges) a step is ~32 launches of a few microseconds each and the eager
+    step is bound by Python's launch path (~1 ms); the replay is one launch.  At config 2 the step is GPU-bound
+    and the graph changes nothing.  The static inputs (features, edge lists) are the tensors of the first call:
+    a different graph object needs a new ``GraphedTrainStep``."""
 
     def __init__(self, model, optimizer, x_dict, edge_index_dict, train_edge_index, interaction_type_tensor,
                  num_users, num_posts):
         if not fused_step.eligible(model, x_dict):
             raise ValueError("GraphedTrainStep needs CUDA inputs and a model the tape-free step accepts")
-        self.model, self.optimizer = model, optimizer
+        dev = x_dict["user"].device
+        super().__init__(model, optimizer, train_edge_index.size(1), dev)
         self.args = (x_dict, edge_index_dict, train_edge_index, interaction_type_tensor, num_users)
         self.num_posts = int(num_posts)
-        dev = x_dict["user"].device
-        self.neg = torch.empty(train_edge_index.size(1), dtype=torch.int64, device=dev)
-        self.neg_ready = torch.cuda.Event(external=True)
         self.side = torch.cuda.Stream(dev)
-        self.graph = self.loss = None
-        self.params, self.grads, self.launches_per_replay = [], [], 0
 
     def matches(self, model, optimizer, x_dict, edge_index_dict, train_edge_index):
         a = self.args
@@ -69,33 +125,10 @@ class GraphedTrainStep:
         return fused_step.loss_and_grads(self.model, x_dict, edge_index_dict, train_edge_index, itt, num_users,
                                          self.neg, neg_ready=self.neg_ready).clone()
 
-    def _capture(self):
-        from . import _lib
-        if _lib.PROF.enabled:
-            raise _lib.TrgError("GraphedTrainStep: per-call event timing (PROF) cannot run inside a graph capture")
-        cur = torch.cuda.current_stream()
-        warm = torch.cuda.Stream(self.neg.device)
-        warm.wait_stream(cur)
-        with torch.cuda.stream(warm):
-            for _ in range(2):            # structures (CSRs), lazy weights, allocator; the optimiser is not stepped
-                self.optimizer.zero_grad(set_to_none=True)
-                self._body()
-        cur.wait_stream(warm)
-        torch.cuda.synchronize()
-        self.optimizer.zero_grad(set_to_none=True)
-        g = torch.cuda.CUDAGraph()
-        n0 = _lib.launch_count()
-        with torch.cuda.graph(g, capture_error_mode="thread_local"):
-            self.loss = self._body()
-        self.launches_per_replay = _lib.launch_count() - n0
-        self.params = [p for p in self.model.parameters() if p.grad is not None]
-        self.grads = [p.grad for p in self.params]
-        self.graph = g
+    def _draw_negatives(self):
+        return torch.randint(0, self.num_posts, (self.neg.numel(),), device=self.neg.device)
 
-    def __call__(self, neg_p=None, return_tensor=False):
-        self.model.train()
-        if neg_p is None:
-            neg_p = torch.randint(0, self.num_posts, (self.neg.numel(),), device=self.neg.device)
+    def _upload(self, neg_p):
         if neg_p.is_cuda:
             self.neg.copy_(neg_p)
             self.neg_ready.record()
@@ -104,13 +137,6 @@ class GraphedTrainStep:
             with torch.cuda.stream(self.side):
                 self.neg.copy_(neg_p, non_blocking=True)
                 self.neg_ready.record(self.side)
-        if self.graph is None:
-            self._capture()
-        self.graph.replay()
-        for p, g in zip(self.params, self.grads):
-            p.grad = g
-        self.optimizer.step()
-        return self.loss if return_tensor else self.loss.item()
 
 
 def train_step(model, optimizer, x_dict, edge_index_dict, train_edge_index, interaction_type_tensor,
