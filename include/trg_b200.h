@@ -188,7 +188,9 @@ int trg_edge_anchor_loss(const int32_t* rowptr, const int32_t* col, const int32_
  * up to 4 (A, W) pairs (user rows: mean_direct, mean_social, x; post rows: mean, x).
  * fp32 inputs are multiplied as 3xTF32 split products on tcgen05 (fp32-accurate), bf16 inputs as
  * kind::f16 with fp32 TMEM accumulation (hidden in {64,128,256}, k_i a multiple of 128 bytes);
- * other shapes take a strict-fp32 FMA kernel.  Workspace: trg_sage_proj_workspace_bytes. */
+ * other shapes take a strict-fp32 FMA kernel.  The bf16 tensor-core path stores alpha_i * W_i as its
+ * bf16 weight operand, so an alpha that is not a power of two rounds that product once (2^-9 relative).
+ * Workspace: trg_sage_proj_workspace_bytes. */
 typedef struct {
   const void* a;      /* [n_rows, k] dtype, row-major, 16B-aligned */
   const void* w;      /* [hidden, k] dtype, row-major (torch Linear.weight layout) */
@@ -205,7 +207,8 @@ int trg_sage_proj_fwd(const trg_proj_term* terms /* host */, int32_t n_terms,
 /* Input-gradient half of the backward of trg_sage_proj_fwd (autograd of F.linear at
  * train_gnn.py:283, needed for layers >= 2):  d_a_i = row_scale_i * ( alpha_i * dZ @ W_i ),
  * dZ[n_rows, hidden] = dOut masked by the ReLU.  row_scale (nullable, fp32 [n_rows]) fuses the
- * 1/deg of the mean aggregation so that K2 is a plain gather-sum.  All k_i must be equal. */
+ * 1/deg of the mean aggregation so that K2 is a plain gather-sum.  All k_i must be equal for the
+ * tensor-core path.  bf16 rounds alpha_i * W_i to bf16 once, as the forward's tensor-core path does. */
 typedef struct {
   const void* w;          /* [hidden, k] dtype */
   int32_t k;
@@ -220,7 +223,7 @@ int trg_sage_proj_bwd_input(const void* dz, const trg_proj_bwd_term* terms /* ho
 /* Weight-gradient half: dW_i = alpha_i * dZ^T @ A_i (reduction over the node rows) and
  * db = column sums of dZ (nullable).  Both operands are consumed MN-major from the row-major
  * tables by tcgen05 (3xTF32 for fp32); per-CTA partials are reduced in a fixed order
- * (deterministic).  Workspace: trg_sage_proj_dw_workspace_bytes(). */
+ * (deterministic).  n_rows = 0 writes dW = 0 and db = 0.  Workspace: trg_sage_proj_dw_workspace_bytes(). */
 typedef struct {
   const void* a;   /* [n_rows, k] dtype */
   int32_t k;

@@ -7,7 +7,8 @@ import truth_recommendation_gnn_b200 as trg
 from oracle import sage as osage
 from oracle import topk as otopk
 from tests.util import (TOL_BF16, TOL_F32, assert_as_accurate_as_fp32, assert_close, assert_close_elementwise,
-                        golden_graph, load_golden, oracle_grads_with_gates, oracle_model, product_gates)
+                        golden_graph, load_golden, oracle_grads_bf16, oracle_grads_with_gates, oracle_model,
+                        product_gates)
 from truth_recommendation_gnn_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -168,20 +169,26 @@ def test_multi_layer_needs_transposed_backward(dev):
         assert_close(a.grad.cpu(), b.grad, 5 * TOL_F32, f"grad {n}")
 
 
-@pytest.mark.parametrize("layers,h,dtype,tol", [(1, 64, torch.float32, 5 * TOL_F32), (2, 128, torch.float32, 5 * TOL_F32),
-                                                (3, 32, torch.float32, 5 * TOL_F32), (2, 128, torch.bfloat16, 3 * TOL_BF16)])
-def test_fused_step_matches_autograd_and_oracle(dev, layers, h, dtype, tol):
+@pytest.mark.parametrize("layers,h,feat,dtype,tol", [
+    (1, 64, 64, torch.float32, 5 * TOL_F32), (2, 128, 128, torch.float32, 5 * TOL_F32),
+    (3, 32, 32, torch.float32, 5 * TOL_F32), (2, 128, 128, torch.bfloat16, 3 * TOL_BF16),
+    (2, 256, 256, torch.float32, 5 * TOL_F32),
+    (3, 256, 256, torch.bfloat16, 3 * TOL_BF16),     # config 4's layer shape
+    (2, 128, 64, torch.float32, 5 * TOL_F32),        # the reference's 64-d features under a wider hidden
+    (2, 128, 64, torch.bfloat16, 3 * TOL_BF16),
+])
+def test_fused_step_matches_autograd_and_oracle(dev, layers, h, feat, dtype, tol):
     """The tape-free step (fused_step.loss_and_grads: ReLU backward and gradient accumulation in
     kernel epilogues) against the autograd path over the same kernels and against the oracle."""
     from truth_recommendation_gnn_b200 import fused_step
     U, P, Ee, Es = 400, 900, 9000, 2500
-    sd = synth.init_state_dict(h, h, layers)
+    sd = synth.init_state_dict(h, feat, layers)
     rnd = (lambda t: t.to(dtype).float())
     neg = synth.synth_neg(P, Ee, 2)
-    g = synth.synth_graph(U, P, Ee, Es, h, seed=11, skew=True)
+    g = synth.synth_graph(U, P, Ee, Es, feat, seed=11, skew=True)
     xr = {k: rnd(v) for k, v in g.x_dict.items()}
     sdr = {k: rnd(v) for k, v in sd.items()}
-    ref = oracle_model(h, layers, sdr)
+    ref = oracle_model(h, layers, sdr, fin=feat)
     gd = g.to(dev)
     xd = {k: v.to(dtype) for k, v in gd.x_dict.items()}
     out = ref(xr, g.edge_index_dict)
@@ -198,10 +205,13 @@ def test_fused_step_matches_autograd_and_oracle(dev, layers, h, dtype, tol):
     assert torch.equal(l_fused, l_auto.detach())              # same forward kernels, same inputs
     ltol = TOL_F32 if dtype == torch.float32 else TOL_BF16
     assert abs(float(l_fused) - float(l_ref)) <= ltol * abs(float(l_ref))
-    g_gated = None
+    g_gated = g_bf16 = None
+    g_copy = synth.SynthGraph(xr, g.edge_index_dict, g.train_edge_index, g.interaction_type_tensor, U, P)
     if dtype == torch.float32:
-        g_copy = synth.SynthGraph(xr, g.edge_index_dict, g.train_edge_index, g.interaction_type_tensor, U, P)
-        _, g_gated, _ = oracle_grads_with_gates(h, layers, sdr, g_copy, neg, product_gates(m_auto, xd, gd.edge_index_dict))
+        _, g_gated, _ = oracle_grads_with_gates(h, layers, sdr, g_copy, neg, product_gates(m_auto, xd, gd.edge_index_dict),
+                                                fin=feat)
+    else:
+        g_bf16 = oracle_grads_bf16(h, layers, sdr, g_copy, neg, fin=feat)
     for (n, a), (_, b), (_, r) in zip(m_fused.named_parameters(), m_auto.named_parameters(), ref.named_parameters()):
         assert a.grad is not None and a.grad.dtype == a.dtype, n
         assert_close(a.grad.float().cpu(), b.grad.float().cpu(), tol, f"fused vs autograd grad {n}")
@@ -212,8 +222,12 @@ def test_fused_step_matches_autograd_and_oracle(dev, layers, h, dtype, tol):
             assert_close(a.grad.cpu(), g_gated[n], tol, f"fused vs oracle grad {n}")
         elif layers == 1 or n.startswith(f"layers.{layers - 1}."):
             # bf16 stores every intermediate gradient table in bf16 and flips ReLU gates near 0: deeper
-            # layers are only checked against the tape path (same storage), the last layer against the oracle
-            assert_close(a.grad.float().cpu(), r.grad, tol, f"fused vs oracle grad {n}")
+            # layers are only checked against the tape path (same storage), the last layer against the oracle.
+            # Where a gradient cancels so far that the oracle's own bf16 run is already more than tol / 2 away
+            # from its fp32 run (measured: the post_update gradients at feat 64 < h 128, 4.0e-2 .. 5.9e-2 on a
+            # B200 and on the CPU alike), the product may be twice that far, no further.
+            bound = max(tol, 2 * osage.rel_err_norm(g_bf16[n], r.grad))
+            assert_close(a.grad.float().cpu(), r.grad, bound, f"fused vs oracle grad {n}")
     # a second call accumulates like loss.backward() does
     g0 = {n: p.grad.clone() for n, p in m_fused.named_parameters()}
     fused_step.loss_and_grads(m_fused, xd, gd.edge_index_dict, gd.train_edge_index, gd.interaction_type_tensor,

@@ -92,12 +92,12 @@ def product_gates(model, x_dict, edge_index_dict):
     return gates
 
 
-def oracle_grads_with_gates(h, layers, sd, g, neg, gates, dtype=torch.float32, kink=1e-5):
+def oracle_grads_with_gates(h, layers, sd, g, neg, gates, dtype=torch.float32, kink=1e-5, fin=None):
     """Gradients of the reference loss (train_gnn.py:259-283) from the oracle with the ReLU gates forced to
     ``gates`` (see ``oracle.sage.forward_gated``), after checking against an fp64 run that those gates differ
     from the exact ones ONLY where the pre-activation is within ``kink`` (relative to the layer's scale) of 0.
     Returns ``(loss, {param name: grad}, n_ambiguous_gates)``."""
-    m64 = oracle_model(h, layers, sd).double()
+    m64 = oracle_model(h, layers, sd, fin).double()
     x64 = {k: v.double() for k, v in g.x_dict.items()}
     with torch.no_grad():
         _, zs = osage.forward_gated(m64, x64, g.edge_index_dict, gates)
@@ -111,9 +111,21 @@ def oracle_grads_with_gates(h, layers, sd, g, neg, gates, dtype=torch.float32, k
                 worst = float(z[wrong].abs().max() / z.abs().max())
                 assert worst <= kink, f"layer {l} {what}: a gate differs where |z| = {worst:.2e} of the scale"
                 n_amb += int(wrong.sum())
-    m = oracle_model(h, layers, sd).to(dtype)
+    m = oracle_model(h, layers, sd, fin).to(dtype)
     out, _ = osage.forward_gated(m, {k: v.to(dtype) for k, v in g.x_dict.items()}, g.edge_index_dict, gates)
     loss = osage.link_loss(out["user"], out["post"], g.train_edge_index[0], g.train_edge_index[1], neg,
                            g.interaction_type_tensor.to(dtype), g.num_users)
     loss.backward()
     return float(loss), {n: p.grad for n, p in m.named_parameters()}, n_amb
+
+
+def oracle_grads_bf16(h, layers, sd, g, neg, fin=None):
+    """Gradients of the reference loss from the oracle run in bf16: parameters, inputs and every intermediate
+    table rounded to bf16 as each op produces it (PyTorch's bf16 CPU ops), the loss taken in fp32 on the bf16
+    embeddings.  Their distance from the fp32 oracle is what bf16 storage alone costs on that input."""
+    m = oracle_model(h, layers, sd, fin).to(torch.bfloat16)
+    out = m({k: v.to(torch.bfloat16) for k, v in g.x_dict.items()}, g.edge_index_dict)
+    loss = osage.link_loss(out["user"].float(), out["post"].float(), g.train_edge_index[0], g.train_edge_index[1],
+                           neg, g.interaction_type_tensor.float(), g.num_users)
+    loss.backward()
+    return {n: p.grad.float() for n, p in m.named_parameters()}

@@ -142,6 +142,12 @@ extern "C" int trg_sage_proj_bwd_weight(const void* dz, const trg_proj_dw_term* 
                   "trg_sage_proj_bwd_weight: term %d needs 16-byte aligned rows", i);
     ks[i] = terms[i].k;
   }
+  if (n_rows == 0) {   // empty sum over rows: dW = 0, db = 0 (a tensor map cannot have a zero extent)
+    for (int i = 0; i < n_terms; ++i)
+      TRG_CUDA(cudaMemsetAsync(terms[i].d_w, 0, (size_t)hidden * terms[i].k * es, st));
+    if (d_bias) TRG_CUDA(cudaMemsetAsync(d_bias, 0, (size_t)hidden * sizeof(float), st));
+    return TRG_OK;
+  }
   if (!force_simt() && tc::proj_dw_eligible(ks, n_terms, hidden, dtype))
     return tc::proj_tc_bwd_weight(dz, terms, n_terms, d_bias, n_rows, hidden, dtype, workspace,
                                   workspace_bytes, st);

@@ -513,7 +513,12 @@ __global__ void __launch_bounds__(256) colsum_simt(const T* __restrict__ dz, lon
 int proj_simt_bwd_weight(const void* dz, const trg_proj_dw_term* terms, int n_terms, float* db,
                          int64_t n_rows, int hidden, int dtype, void* ws, size_t ws_bytes,
                          cudaStream_t st) {
-  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(grid_sms(), (n_rows + 63) / 64));
+  // one [hidden, k] partial per CTA: wide terms (k up to 512) take fewer CTAs so that the widest
+  // term's partials fit the workspace
+  int kmax = 1;
+  for (int t = 0; t < n_terms; ++t) kmax = std::max(kmax, terms[t].k);
+  const int64_t fit = (int64_t)(ws_bytes / ((size_t)hidden * kmax * sizeof(float)));
+  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>({(int64_t)grid_sms(), (n_rows + 63) / 64, fit}));
   const int64_t rows_per_cta = (n_rows + grid - 1) / grid;
   float* partial = reinterpret_cast<float*>(ws);
   for (int t = 0; t <= n_terms; ++t) {
