@@ -11,7 +11,8 @@
  *  - no ownership transfer: all buffers including workspaces are allocated by the caller;
  *  - stateless, asynchronous on the given stream (a cudaStream_t passed as void*), no host
  *    synchronisation inside, re-entrant across streams and threads;
- *  - dtype: TRG_F32 (fp32 storage) or TRG_BF16 (bf16 storage, fp32 accumulation);
+ *  - dtype: TRG_F32 (fp32 storage) or TRG_BF16 (bf16 storage, fp32 accumulation); TRG_F8E4M3 (e4m3
+ *    bytes, fp32 accumulation) is accepted by trg_score_topk / trg_score_topk_excluding only;
  *  - row widths (F, H) must make a row a multiple of 16 bytes (F % 4 == 0 for fp32,
  *    F % 8 == 0 for bf16) and tables must be 16-byte aligned;
  *  - edge counts must be < 2^31 per relation; node ids are stored as int32 in the CSR.
@@ -28,7 +29,7 @@ extern "C" {
 
 #define TRG_ABI_VERSION 4
 
-enum { TRG_F32 = 0, TRG_BF16 = 1 };
+enum { TRG_F32 = 0, TRG_BF16 = 1, TRG_F8E4M3 = 2 /* trg_score_topk(_excluding) only */ };
 enum {
   TRG_OK = 0,
   TRG_E_ARG = 1,        /* bad argument (null pointer, unsupported width, size overflow) */
@@ -268,6 +269,21 @@ int trg_score_topk_excluding(const void* q /* [B, H] */, const void* cat /* [P, 
 int trg_topk_merge(const float* vals_in /* [B, n_lists*k_in] */, const int64_t* ids_in,
                    int64_t n_query, int32_t n_lists, int32_t k_in, int32_t k_out,
                    float* vals_out, int64_t* ids_out, void* stream);
+
+/* Exact re-ranking of per-query candidate lists (the second stage of a top-k whose first stage ran on
+ * TRG_F8E4M3 copies of the tables).  dtype TRG_F32 or TRG_BF16; q [B, H] and table [P, H] row-major and
+ * 16-byte aligned; cand_ids int64 [B, n_cand] GLOBAL post ids (the id space of ids_out: local + id_offset).
+ * Candidate g of query b, when id_offset <= g < id_offset + n_table, scores
+ *     s = 0; for h = 0 .. H-1: s = fmaf(float(q[b][h]), float(table[g - id_offset][h]), s)
+ * -- the order of trg_score_topk's fp32 kernel, so an fp32 table gives its scores bit for bit.  Candidates
+ * with id -1 or outside that range are skipped (never read).  Candidates are expected to be distinct.
+ * The top k_out = min(k, n_cand) <= 128 of each row under (score desc, id asc) are written to
+ * vals_out / ids_out [B, k_out]; a row with fewer valid candidates is padded at its tail with (-inf, -1). */
+size_t trg_rescore_topk_workspace_bytes(int64_t n_query, int32_t n_cand);
+int trg_rescore_topk(const void* q /* [B, H] */, const void* table /* [P, H] */, int64_t n_query, int64_t n_table,
+                     int32_t hidden, int dtype, const int64_t* cand_ids /* [B, n_cand] */, int32_t n_cand,
+                     int64_t id_offset, int32_t k, float* vals_out /* [B, k_out] */,
+                     int64_t* ids_out /* [B, k_out] */, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -9,6 +9,7 @@ from . import _lib, dist, dist_fused, fused_step, graph_io, synth  # noqa: F401
 from .functional import (link_bce_loss, sage_mean_aggregate, score_topk, topk_merge)  # noqa: F401
 from .graph import CSR, RelationGraph, build_csr, clear_cache, relation_graph  # noqa: F401
 from .exclusion import ExclusionIndex  # noqa: F401
+from .fp8 import Fp8Catalogue  # noqa: F401
 from .nn import (REL_DIRECT, REL_ENGAGE, REL_SOCIAL, Linear, SAGEConv, StackedWeightedRGCN,  # noqa: F401
                  WeightedRGCN)
 from .evaluation import embed_cold_users, evaluate, recommend_cold_users  # noqa: F401

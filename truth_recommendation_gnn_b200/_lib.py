@@ -13,7 +13,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libtrg_b200.so")
 
-TRG_F32, TRG_BF16 = 0, 1
+TRG_F32, TRG_BF16, TRG_F8E4M3 = 0, 1, 2   # TRG_F8E4M3: trg_score_topk(_excluding) only
 ABI_VERSION = 4    # TRG_ABI_VERSION of include/trg_b200.h
 
 _vp, _i64, _i32, _sz, _int = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_size_t, ctypes.c_int
@@ -70,6 +70,9 @@ SIGNATURES = {
     "trg_score_topk_excluding": (_int, [_vp, _vp, _i64, _i64, _i32, _int, _i32, _i64, _vp, _vp, _vp, _vp, _vp,
                                         _vp, _sz, _vp]),
     "trg_topk_merge": (_int, [_vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "trg_rescore_topk_workspace_bytes": (_sz, [_i64, _i32]),
+    "trg_rescore_topk": (_int, [_vp, _vp, _i64, _i64, _i32, _int, _vp, _i32, _i64, _i32, _vp, _vp, _vp, _sz,
+                                _vp]),
 }
 
 _lib = None

@@ -559,13 +559,15 @@ int make_tmap_2d(CUtensorMap* map, const void* base, int dtype, uint64_t rows, u
     set_error("cuTensorMapEncodeTiled entry point not available");
     return TRG_E_CUDA;
   }
-  const int es = dtype == TRG_BF16 ? 2 : 4;
+  const int es = dtype == TRG_BF16 ? 2 : dtype == TRG_F8E4M3 ? 1 : 4;
+  const CUtensorMapDataType dt = dtype == TRG_BF16     ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                                 : dtype == TRG_F8E4M3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8
+                                                       : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   cuuint64_t gdim[2] = {cols, rows};
   cuuint64_t gstride[1] = {ld_elems * es};
   cuuint32_t box[2] = {(cuuint32_t)(128 / es), box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, dtype == TRG_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
-                   2, const_cast<void*>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+  CUresult r = enc(map, dt, 2, const_cast<void*>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {

@@ -296,7 +296,7 @@ int choose_splits(int64_t n_query, int64_t n_cat, int64_t* tiles_per_split) {
 namespace tc {
 bool score_tc_eligible(int hidden, int dtype, int k);
 size_t score_tc_workspace_bytes(int64_t n_query, int64_t n_cat, int hidden, int k);
-int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat, int hidden, int k,
+int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat, int hidden, int dtype, int k,
                   int64_t id_offset, const int32_t* excl_rowptr, const int32_t* excl_ids,
                   const int64_t* query_rows, float* vals_out, int64_t* ids_out, void* ws, size_t ws_bytes,
                   cudaStream_t st);
@@ -323,7 +323,8 @@ extern "C" size_t trg_score_topk_workspace_bytes(int64_t n_query, int64_t n_cat,
   const int64_t kk = std::min<int64_t>(k, n_cat);
   const size_t simt = align_up((size_t)n_query * splits * kk * 4, 256) +
                       align_up((size_t)n_query * splits * kk * 8, 256);
-  // dtype is not part of this query: size for whichever kernel (fp32 FMA / bf16 tcgen05) needs more
+  // dtype is not part of this query: size for whichever kernel (fp32 FMA / bf16 or e4m3 tcgen05) needs more;
+  // the tcgen05 workspace depends on n_query only, so every dtype's need is covered
   size_t tcb = 0;
   if (hidden % 64 == 0 && hidden <= 256 && kk <= 128)
     tcb = tc::score_tc_workspace_bytes(n_query, n_cat, hidden, (int)kk);
@@ -360,13 +361,16 @@ static int score_topk_impl(const char* fn, const void* q, const void* cat, int64
   TRG_CHECK_ARG(!excl_rowptr || excl_ids, "%s: excl_ids must be non-NULL when excl_rowptr is given", fn);
   const int kk = (int)std::min<int64_t>(k, n_cat);
   TRG_CHECK_ARG(kk <= kMaxK, "%s: k=%d > %d is not supported", fn, kk, kMaxK);
-  if (dtype == TRG_BF16) {
+  if (dtype == TRG_BF16 || dtype == TRG_F8E4M3) {   // tcgen05 only: there is no FMA form for e4m3
     if (!tc::score_tc_eligible(hidden, dtype, kk)) {
-      set_error("%s(bf16): hidden=%d k=%d unsupported: hidden must be in {64,128,192,256}, k <= 128, and the query block (256*hidden B) + the per-row lists (1 KiB*k) + two catalogue stages must fit in 227 KiB of shared memory", fn, hidden, kk);
+      if (dtype == TRG_BF16)
+        set_error("%s(bf16): hidden=%d k=%d unsupported: hidden must be in {64,128,192,256}, k <= 128, and the query block (256*hidden B) + the per-row lists (1 KiB*k) + two catalogue stages must fit in 227 KiB of shared memory", fn, hidden, kk);
+      else
+        set_error("%s(e4m3): hidden=%d k=%d unsupported: hidden must be 128 or 256 and k <= 128", fn, hidden, kk);
       return TRG_E_UNSUPPORTED;
     }
-    return tc::score_topk_tc(q, cat, n_query, n_cat, hidden, kk, id_offset, excl_rowptr, excl_ids, query_rows,
-                             vals_out, ids_out, workspace, workspace_bytes, st);
+    return tc::score_topk_tc(q, cat, n_query, n_cat, hidden, dtype, kk, id_offset, excl_rowptr, excl_ids,
+                             query_rows, vals_out, ids_out, workspace, workspace_bytes, st);
   }
   if (dtype != TRG_F32) {
     set_error("%s: unknown dtype %d", fn, dtype);

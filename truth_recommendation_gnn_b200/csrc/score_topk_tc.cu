@@ -1,4 +1,4 @@
-// K5 (tcgen05 form) -- bf16 score contraction + streaming top-k on the tensor cores.
+// K5 (tcgen05 form) -- bf16 or e4m3 score contraction + streaming top-k on the tensor cores.
 //
 // Replaces  scores = torch.mm(user_emb, known_post_emb.T); torch.topk(scores, min(K, n))
 // (inference.py:427-428) for batched queries against a large catalogue (BASELINE config 5:
@@ -8,8 +8,8 @@
 // One persistent CTA (16 warps) per SM; work = (catalogue chunk, 128-query block) items, chunk-major.
 //   warp 0      TMA: the item's query block (all k-blocks resident), then catalogue tiles [128 posts x H]
 //               through an mbarrier ring (SWIZZLE_128B, K-major)
-//   warp 1      one thread issues tcgen05.mma kind::f16 (bf16 in, fp32 accumulate), accumulators
-//               double-buffered in TMEM columns [0, 256)
+//   warp 1      one thread issues tcgen05.mma kind::f16 (bf16 in) or kind::f8f6f4 (e4m3 in), fp32
+//               accumulate, accumulators double-buffered in TMEM columns [0, 256)
 //   warps 4-11  SCAN: lane r of a quarter owns query row r (= TMEM lane r), two warps per quarter take 64
 //               columns each: tcgen05.ld, one max tree + one warp vote against the row's K-th best; a lane
 //               with a candidate copies its 64 scores into a hand-off slot
@@ -19,6 +19,9 @@
 //               of an item, rank merge of the item's lists into the rows' GLOBAL lists (the result buffer)
 //               under one lock per row
 // Tensor-bound: 2*B*P*H flops against 2*P*H bytes of catalogue (AI = B = 4096 flop/B).
+// E4M3: one 128-byte k-block holds 128 elements instead of 64 and an MMA covers K = 32 instead of 16, so
+// every k-block is issued exactly as in bf16 (4 MMAs, +32 bytes each) over half as many k-blocks: half the
+// catalogue bytes and half the tensor time per tile.  Everything after the accumulator is unchanged.
 // History and measurements of the earlier forms (v1: selection on the accumulator-reading warps; v2: scan /
 // helper split; v4: candidates filtered in registers -- slower at 50M posts, dropped): profiles/README.md.
 #include <algorithm>
@@ -44,7 +47,7 @@ struct ScoreTcParams {
   CUtensorMap c_map;
   long long n_query, n_cat, id_offset;
   long long tiles_per_split;
-  int k, n_splits, kblocks;   // kblocks = H / 64
+  int k, n_splits, kblocks;   // kblocks = H * bytes per element / 128
   int dbg;                    // ablation switches, TRG_DEBUG builds only (TRG_TOPK_DBG): 1 = no selection, 2 = no tcgen05.ld either, 4 = no MMA
   int* thr_shared;            // [B] ordered-int keys of the best published K-th score per query row
   int* locks;                 // [B] one lock per query row's global list
@@ -321,10 +324,12 @@ __device__ __forceinline__ float merge_into_global(const ScoreTcParams& p, long 
 // excluded post ever enters a list -- per-item lists, flushed global lists, row_thr and thr_shared then only
 // ever hold admissible posts, and every threshold below stays the exact K-th best of what may be returned.
 // The scan warps' filter (max against those thresholds) remains a superset test and is unchanged.
-template <int NS, bool EXCL>
+// E4M3: both operands are e4m3 bytes (kind::f8f6f4); otherwise bf16 (kind::f16).
+template <int NS, bool EXCL, bool E4M3>
 __global__ void __launch_bounds__(512, 1)
     score_topk_tc3_kernel(const __grid_constant__ ScoreTcParams p, int n_stages) {
   constexpr int N = kTileN2;
+  constexpr int kElemsPerKb = E4M3 ? 128 : 64;   // elements in one 128-byte k-block
   constexpr int kSub = N / NS;
   constexpr int kChains = 8;
   constexpr int kQStride = kQCap2 + 1;
@@ -398,14 +403,16 @@ __global__ void __launch_bounds__(512, 1)
         if (seg > 0) mbar_wait_backoff(smem_u32(q_free), (seg - 1) & 1);    // the previous segment's MMAs are done with Q
         mbar_arrive_expect_tx(smem_u32(q_full), (uint32_t)q_bytes);
         for (int kb = 0; kb < p.kblocks; ++kb)
-          tma_load_2d(smem_u32(q_smem + kb * kQRows * 128), &p.q_map, smem_u32(q_full), kb * 64, (int)(sg.qb * kQRows));
+          tma_load_2d(smem_u32(q_smem + kb * kQRows * 128), &p.q_map, smem_u32(q_full), kb * kElemsPerKb,
+                      (int)(sg.qb * kQRows));
         for (int t = 0; t < sg.n_tiles * kSub; ++t) {
           mbar_wait_backoff(smem_u32(&empty[stage]), phase ^ 1);
           const uint32_t fb = smem_u32(&full[stage]);
           mbar_arrive_expect_tx(fb, (uint32_t)stage_bytes);
           const int row = (int)(sg.tile0 * N + (long long)t * NS);
           for (int kb = 0; kb < p.kblocks; ++kb)
-            tma_load_2d(smem_u32(ring + (size_t)stage * stage_bytes + kb * NS * 128), &p.c_map, fb, kb * 64, row);
+            tma_load_2d(smem_u32(ring + (size_t)stage * stage_bytes + kb * NS * 128), &p.c_map, fb, kb * kElemsPerKb,
+                        row);
           if (++stage == n_stages) { stage = 0; phase ^= 1; }
         }
         ++seg;
@@ -413,7 +420,7 @@ __global__ void __launch_bounds__(512, 1)
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(kFmtBF16, 0, 0, kQRows, NS);
+      constexpr uint32_t idesc = make_idesc(E4M3 ? kFmtE4M3 : kFmtBF16, 0, 0, kQRows, NS);
       int stage = 0, acc = 0;
       uint32_t phase = 0, acc_phase = 0, seg = 0;
       long long item = blockIdx.x;
@@ -432,8 +439,12 @@ __global__ void __launch_bounds__(512, 1)
               const uint64_t cd = make_smem_desc_sw128(smem_u32(ring + (size_t)stage * stage_bytes + kb * NS * 128), 0, 1024);
               if (!(TRG_TOPK_DBG(p) & 4)) {
 #pragma unroll
-                for (int k = 0; k < 4; ++k)
-                  umma_ss<false>(d, qd + (uint64_t)(2 * k), cd + (uint64_t)(2 * k), idesc, (kb | k) ? 1u : 0u);
+                for (int k = 0; k < 4; ++k) {
+                  if constexpr (E4M3)
+                    umma_ss_f8f6f4(d, qd + (uint64_t)(2 * k), cd + (uint64_t)(2 * k), idesc, (kb | k) ? 1u : 0u);
+                  else
+                    umma_ss<false>(d, qd + (uint64_t)(2 * k), cd + (uint64_t)(2 * k), idesc, (kb | k) ? 1u : 0u);
+                }
               }
             }
             umma_commit(smem_u32(&empty[stage]));
@@ -806,10 +817,14 @@ __global__ void __launch_bounds__(512, 1)
 int make_tmap_2d(CUtensorMap* map, const void* base, int dtype, uint64_t rows, uint64_t cols,
                  uint64_t ld_elems, uint32_t box_rows);
 
-bool score_tc_fits(int hidden);
+bool score_tc_fits(int row_bytes);
+// bf16: H in {64, 128, 192, 256}; e4m3: H in {128, 256} (a 64-byte row would need SWIZZLE_64B)
 bool score_tc_eligible(int hidden, int dtype, int k) {
-  return dtype == TRG_BF16 && hidden % 64 == 0 && hidden >= 64 && hidden <= 256 && k >= 1 && k <= 128 &&
-         score_tc_fits(hidden) && get_encode_tiled() != nullptr;
+  const bool shape = dtype == TRG_BF16     ? hidden % 64 == 0 && hidden >= 64 && hidden <= 256
+                     : dtype == TRG_F8E4M3 ? hidden == 128 || hidden == 256
+                                           : false;
+  const int row_bytes = hidden * (dtype == TRG_BF16 ? 2 : 1);
+  return shape && k >= 1 && k <= 128 && score_tc_fits(row_bytes) && get_encode_tiled() != nullptr;
 }
 
 constexpr int kSmemLimit = 227 * 1024;
@@ -834,24 +849,25 @@ static int score_tc_partition(int64_t n_query, int64_t n_cat, long long* tiles_p
   return (int)std::min<int64_t>(sms, s * q_blocks);
 }
 
-static int fixed_smem3(int hidden) {
-  return (hidden / 64) * kQRows * 128 + 8 * kSlotRing3 * kSlotWords3 * 4 + 4 * 128 * 8 + kQRows * (kQCap2 + 1) * 8 +
+// row_bytes = H * bytes per element: one query / catalogue row, a whole number of 128-byte k-blocks
+static int fixed_smem3(int row_bytes) {
+  return (row_bytes / 128) * kQRows * 128 + 8 * kSlotRing3 * kSlotWords3 * 4 + 4 * 128 * 8 + kQRows * (kQCap2 + 1) * 8 +
          4 * 128 * 12 /*global-list scratch*/ + kQRows * 12 + 128 + 8 + 1024 + 512;
 }
 // deep ring first (TMA latency x bandwidth), widest stage that allows it
-static ScoreCfg pick_cfg3(int hidden) {
-  const int fixed = fixed_smem3(hidden);
+static ScoreCfg pick_cfg3(int row_bytes) {
+  const int fixed = fixed_smem3(row_bytes);
   const int force_ns = debug_env_int("TRG_TOPK_NS", 0);      // TRG_DEBUG builds only: stage width A/B
   for (int min_stages : {4, 2})
     for (int ns : {kTileN2, kTileN2 / 2}) {
       if (force_ns && ns != force_ns) continue;
-      const int stage = (hidden / 64) * ns * 128;
+      const int stage = (row_bytes / 128) * ns * 128;
       const int stages = std::min(8, (kSmemLimit - fixed) / stage);
       if (stages >= min_stages) return {ns, stages, fixed + stages * stage};
     }
   return {0, 0, 0};
 }
-bool score_tc_fits(int hidden) { return pick_cfg3(hidden).ns > 0; }
+bool score_tc_fits(int row_bytes) { return pick_cfg3(row_bytes).ns > 0; }
 
 size_t score_tc_workspace_bytes(int64_t n_query, int64_t n_cat, int hidden, int k) {
   (void)n_cat; (void)hidden; (void)k;
@@ -876,15 +892,15 @@ __global__ void pads_to_minus_one(long long* ids, long long n) {
     if (ids[i] == kPadIdTc) ids[i] = -1;
 }
 
-template <int NS, bool EXCL>
+template <int NS, bool EXCL, bool E4M3>
 static int launch_score3(const ScoreTcParams& p, int grid, int smem, int n_stages, cudaStream_t st) {
   static SmemAttrState attr;
-  TRG_CUDA(ensure_dyn_smem(score_topk_tc3_kernel<NS, EXCL>, smem, attr));
-  score_topk_tc3_kernel<NS, EXCL><<<grid, 512, smem, st>>>(p, n_stages);
+  TRG_CUDA(ensure_dyn_smem(score_topk_tc3_kernel<NS, EXCL, E4M3>, smem, attr));
+  score_topk_tc3_kernel<NS, EXCL, E4M3><<<grid, 512, smem, st>>>(p, n_stages);
   return TRG_OK;
 }
 
-int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat, int hidden, int k,
+int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat, int hidden, int dtype, int k,
                   int64_t id_offset, const int32_t* excl_rowptr, const int32_t* excl_ids,
                   const int64_t* query_rows, float* vals_out, int64_t* ids_out, void* ws, size_t ws_bytes,
                   cudaStream_t st) {
@@ -893,17 +909,19 @@ int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat
     set_error("trg_score_topk: workspace %zu < required %zu", ws_bytes, need);
     return TRG_E_WORKSPACE;
   }
-  const ScoreCfg cfg = pick_cfg3(hidden);
+  const bool e4m3 = dtype == TRG_F8E4M3;
+  const int row_bytes = hidden * (e4m3 ? 1 : 2);
+  const ScoreCfg cfg = pick_cfg3(row_bytes);
   if (cfg.ns == 0) {
-    set_error("trg_score_topk(bf16): hidden=%d k=%d does not fit in shared memory", hidden, k);
+    set_error("trg_score_topk(%s): hidden=%d k=%d does not fit in shared memory", e4m3 ? "e4m3" : "bf16", hidden, k);
     return TRG_E_UNSUPPORTED;
   }
   ScoreTcParams p{};
-  int rc = make_tmap_2d(&p.q_map, q, TRG_BF16, (uint64_t)n_query, hidden, hidden, kQRows);
+  int rc = make_tmap_2d(&p.q_map, q, dtype, (uint64_t)n_query, hidden, hidden, kQRows);
   if (rc) return rc;
-  rc = make_tmap_2d(&p.c_map, cat, TRG_BF16, (uint64_t)n_cat, hidden, hidden, cfg.ns);
+  rc = make_tmap_2d(&p.c_map, cat, dtype, (uint64_t)n_cat, hidden, hidden, cfg.ns);
   if (rc) return rc;
-  p.n_query = n_query; p.n_cat = n_cat; p.id_offset = id_offset; p.k = k; p.kblocks = hidden / 64;
+  p.n_query = n_query; p.n_cat = n_cat; p.id_offset = id_offset; p.k = k; p.kblocks = row_bytes / 128;
   p.dbg = debug_env_int("TRG_TOPK_DBG", 0);
   const int grid = score_tc_partition(n_query, n_cat, &p.tiles_per_split, &p.n_splits);
   p.thr_shared = reinterpret_cast<int*>(ws);
@@ -920,13 +938,19 @@ int score_topk_tc(const void* q, const void* cat, int64_t n_query, int64_t n_cat
   count_launch();
   // the EXCL = false instantiations come first: the compiler then emits them instruction for instruction as
   // the kernel was before exclusions existed (instantiated after the EXCL ones, the NS = 64 form came out
-  // with a different register assignment)
-  if (!excl)
-    rc = cfg.ns == kTileN2 ? launch_score3<kTileN2, false>(p, grid, cfg.smem, cfg.stages, st)
-                           : launch_score3<kTileN2 / 2, false>(p, grid, cfg.smem, cfg.stages, st);
+  // with a different register assignment); the e4m3 ones come after every bf16 one for the same reason
+  if (!e4m3 && !excl)
+    rc = cfg.ns == kTileN2 ? launch_score3<kTileN2, false, false>(p, grid, cfg.smem, cfg.stages, st)
+                           : launch_score3<kTileN2 / 2, false, false>(p, grid, cfg.smem, cfg.stages, st);
+  else if (!e4m3)
+    rc = cfg.ns == kTileN2 ? launch_score3<kTileN2, true, false>(p, grid, cfg.smem, cfg.stages, st)
+                           : launch_score3<kTileN2 / 2, true, false>(p, grid, cfg.smem, cfg.stages, st);
+  else if (!excl)
+    rc = cfg.ns == kTileN2 ? launch_score3<kTileN2, false, true>(p, grid, cfg.smem, cfg.stages, st)
+                           : launch_score3<kTileN2 / 2, false, true>(p, grid, cfg.smem, cfg.stages, st);
   else
-    rc = cfg.ns == kTileN2 ? launch_score3<kTileN2, true>(p, grid, cfg.smem, cfg.stages, st)
-                           : launch_score3<kTileN2 / 2, true>(p, grid, cfg.smem, cfg.stages, st);
+    rc = cfg.ns == kTileN2 ? launch_score3<kTileN2, true, true>(p, grid, cfg.smem, cfg.stages, st)
+                           : launch_score3<kTileN2 / 2, true, true>(p, grid, cfg.smem, cfg.stages, st);
   if (rc) return rc;
   count_launch();
   if (excl) {

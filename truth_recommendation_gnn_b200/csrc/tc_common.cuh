@@ -150,6 +150,16 @@ __device__ __forceinline__ void umma_ss(uint32_t tmem_d, uint64_t adesc, uint64_
         : "memory");
   }
 }
+// D[tmem] (+)= A[smem] * B[smem] with 8-bit operands (kind::f8f6f4; the idesc's a/b formats say which):
+// K = 32 elements per instruction, i.e. the same 32 bytes of a 128-byte swizzle row as a kind::f16 MMA
+__device__ __forceinline__ void umma_ss_f8f6f4(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
+                                               uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // D[tmem] (+)= A[tmem] * B[smem]: the A operand (M = 128 lanes x K 32-bit columns) is read from
 // tensor memory, so it costs no shared-memory bandwidth (a 128x128x8 tf32 MMA otherwise reads
 // 4 KB of A + 4 KB of B per 64 clocks = the whole 128 B/clk of the SM's shared memory).
@@ -237,13 +247,15 @@ __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t smem_addr, uin
   return d;
 }
 // Instruction descriptor (cute::UMMA::InstrDescriptor): c_format [4,6) = 1 (F32);
-// a_format [7,10), b_format [10,13): 0 F16, 1 BF16, 2 TF32; a_major bit 15, b_major bit 16
+// a_format [7,10), b_format [10,13): 0 F16, 1 BF16, 2 TF32 (kind::f16 / tf32), 0 E4M3 (kind::f8f6f4);
+// a_major bit 15, b_major bit 16
 // (0 = K-major, 1 = MN-major); n_dim [17,23) = N >> 3; m_dim [24,29) = M >> 4.
 __host__ __device__ constexpr uint32_t make_idesc(int fmt, int a_mn_major, int b_mn_major, int m, int n) {
   return (1u << 4) | ((uint32_t)fmt << 7) | ((uint32_t)fmt << 10) | ((uint32_t)a_mn_major << 15) |
          ((uint32_t)b_mn_major << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 constexpr int kFmtBF16 = 1, kFmtTF32 = 2;
+constexpr int kFmtE4M3 = 0;   // under kind::f8f6f4
 
 // ---- host: TMA tensor maps through the driver entry point (no link-time libcuda dependency) ----
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -252,6 +264,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapFloatOOBfill);
 EncodeTiledFn get_encode_tiled();
 // 2-D row-major [rows, cols] matrix, box = [box_rows, 128 bytes of columns], SWIZZLE_128B.
+// dtype TRG_F32 / TRG_BF16 / TRG_F8E4M3 (bytes; out-of-bounds boxes fill with zero bytes = e4m3 +0).
 int make_tmap_2d(CUtensorMap* map, const void* base, int dtype, uint64_t rows, uint64_t cols,
                  uint64_t ld_elems, uint32_t box_rows);
 // 3-D view (32-element column chunk, rows, column chunk index) for MN-major operands.

@@ -9,7 +9,7 @@ import ctypes
 
 import torch
 
-from . import _lib
+from . import _lib, fp8
 from .graph import CSR, RelationGraph, build_csr
 
 
@@ -526,18 +526,28 @@ def fused_projection(terms, bias, relu=True, row_scales=None):
 # ------------------------------------------------------------------------------------------
 # K5: score contraction + top-k (inference.py:427-428)
 # ------------------------------------------------------------------------------------------
-def score_topk(q: torch.Tensor, cat: torch.Tensor, k: int, id_offset: int = 0, exclude=None, rows=None):
+def score_topk(q: torch.Tensor, cat, k: int, id_offset: int = 0, exclude=None, rows=None):
     """``torch.topk(torch.mm(q, cat.T), min(k, len))`` without materialising the scores.
     Returns ``(values[B,k'] fp32 descending, ids[B,k'] int64)`` under (score desc, id asc).
 
     ``exclude``: an ``ExclusionIndex``; query ``b`` then never gets a post id of exclusion row
     ``rows[b]`` (``rows``: int64 ``[B]`` on the device, each in ``[0, exclude.num_rows)``; default: row
     ``b``).  A query with fewer than ``k'`` admissible posts is padded at its tail with
-    ``(-inf, -1)``.  ``exclude=None`` is exactly the call without exclusions."""
-    lib = _lib.load()
+    ``(-inf, -1)``.  ``exclude=None`` is exactly the call without exclusions.
+
+    ``cat`` may be an ``fp8.Fp8Catalogue``: the posts are then selected from its e4m3 copy and re-ranked
+    exactly from its dense table (``fp8.score_topk``; ``q`` must have the table's dtype, ``k <= 128``)."""
+    if isinstance(cat, fp8.Fp8Catalogue):
+        return fp8.score_topk(q, cat, k, id_offset, exclude=exclude, rows=rows)
     if q.dim() == 1:
         q = q.unsqueeze(0)
-    q, cat = q.contiguous(), cat.contiguous()
+    return _score_topk_native(q.contiguous(), cat.contiguous(), k, id_offset, exclude, rows)
+
+
+def _score_topk_native(q, cat, k, id_offset, exclude, rows, code=None):
+    """``trg_score_topk(_excluding)``; ``code``: the tables' dtype code (default: that of ``q.dtype``; e4m3
+    tables pass ``TRG_F8E4M3``)."""
+    lib = _lib.load()
     b, h = q.shape
     p = cat.size(0)
     kk = min(int(k), p)
@@ -558,13 +568,14 @@ def score_topk(q: torch.Tensor, cat: torch.Tensor, k: int, id_offset: int = 0, e
         return vals, ids
     ws_bytes = int(lib.trg_score_topk_workspace_bytes(b, p, h, kk))
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=q.device)
+    code = _lib.dtype_code(q.dtype) if code is None else code
     if exclude is None:
         _lib.call("trg_score_topk", 2 * b * p * h, lib.trg_score_topk,  # "bytes" slot carries flops here
-                  _lib.ptr(q), _lib.ptr(cat), b, p, h, _lib.dtype_code(q.dtype), kk, int(id_offset),
+                  _lib.ptr(q), _lib.ptr(cat), b, p, h, code, kk, int(id_offset),
                   _lib.ptr(vals), _lib.ptr(ids), _lib.ptr(ws), ws_bytes, _lib.stream())
     else:
         _lib.call("trg_score_topk_excluding", 2 * b * p * h, lib.trg_score_topk_excluding,
-                  _lib.ptr(q), _lib.ptr(cat), b, p, h, _lib.dtype_code(q.dtype), kk, int(id_offset),
+                  _lib.ptr(q), _lib.ptr(cat), b, p, h, code, kk, int(id_offset),
                   # an index without any id: every row is empty and no id is read, but the pointer must be valid
                   _lib.ptr(exclude.rowptr), _lib.ptr(exclude.ids if exclude.nnz else exclude.rowptr), _lib.ptr(rows),
                   _lib.ptr(vals), _lib.ptr(ids), _lib.ptr(ws), ws_bytes, _lib.stream())
