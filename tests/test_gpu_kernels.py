@@ -1,6 +1,7 @@
 """GPU parity tests, kernel level: every C-ABI entry point against the CPU oracle on the same
 seeded inputs.  Bit-exact for integer / index work and for the fp32 CSR-order mean; 1e-5
-relative for other fp32 results; 1e-2 for bf16 storage (fp32 accumulate)."""
+relative for other fp32 results; 1e-2 for bf16 storage (fp32 accumulate).  The gather-reduce
+kernels at every form and epilogue, and the row-finish kernels, are in test_gpu_gather.py."""
 import pytest
 import torch
 
@@ -175,53 +176,6 @@ def test_agg_bwd_skipped_for_leaf_features(dev):
     w = torch.randn(64, 64, device=dev, requires_grad=True)
     (trg.sage_mean_aggregate(x.to(dev), rel) @ w).sum().backward()
     assert rel._bwd is None and w.grad is not None
-
-
-# ------------------------------------------------------------------------------------ wsum
-def test_gather_wsum(dev):
-    x, ei = _agg_case(200, 300, 3000, 64, 17)
-    coef = torch.randn(3000, generator=torch.Generator().manual_seed(2))
-    exp = torch.zeros(300, 64, dtype=torch.float64).index_add_(
-        0, ei[1], coef.double()[:, None] * x.double()[ei[0]])
-    csr = trg.RelationGraph(ei.to(dev), 200, 300).fwd
-    scale = torch.tensor([0.5], device=dev)
-    out = Fn.gather_wsum(csr, coef.to(dev), x.to(dev), scale=scale)
-    assert_close(out.cpu(), 0.5 * exp, TOL_F32, "wsum")
-    Fn.gather_wsum(csr, coef.to(dev), x.to(dev), scale=None, out=out, accumulate=True)
-    assert_close(out.cpu(), 1.5 * exp, TOL_F32, "wsum accumulate")
-
-
-@pytest.mark.parametrize("f,dtype,tol,long_rows", [(128, torch.float32, TOL_F32, False), (64, torch.float32, TOL_F32, False),
-                                                   (16, torch.float32, TOL_F32, False), (8, torch.float32, TOL_F32, False),
-                                                   (128, torch.float32, TOL_F32, True), (128, torch.bfloat16, TOL_BF16, False)])
-def test_gather_epilogue_accumulate_and_relu_gate(dev, f, dtype, tol, long_rows, monkeypatch):
-    """accumulate + relu_of epilogues of K2 / wsum (the fused ReLU backward and gradient
-    accumulation of fused_step): out = where(act > 0, base + gather_sum, 0)."""
-    if long_rows:
-        from truth_recommendation_gnn_b200 import graph as G
-        monkeypatch.setattr(G, "LONG_ROW_THRESHOLD", 64)
-    x, ei = _agg_case(300, 200, 6000, f, 77 + f, skew=True)
-    gen = torch.Generator().manual_seed(9)
-    x = x.to(dtype).float()
-    base = torch.randn(200, f, generator=gen).to(dtype).float()
-    act = torch.relu(torch.randn(200, f, generator=gen)).to(dtype).float()
-    coef = torch.randn(6000, generator=gen)
-    csr = trg.RelationGraph(ei.to(dev), 300, 200).fwd
-    s_plain = torch.zeros(200, f, dtype=torch.float64).index_add_(0, ei[1], x.double()[ei[0]])
-    s_coef = torch.zeros(200, f, dtype=torch.float64).index_add_(0, ei[1], coef.double()[:, None] * x.double()[ei[0]])
-    xd, actd = x.to(dev).to(dtype), act.to(dev).to(dtype)
-    for what, run, ssum in (
-            ("agg_bwd", lambda o, **kw: Fn.sage_agg_bwd(csr, None, xd, out=o, **kw), s_plain),
-            ("wsum", lambda o, **kw: Fn.gather_wsum(csr, coef.to(dev), xd, out=o, **kw), s_coef)):
-        out = run(base.to(dev).to(dtype).clone(), accumulate=True)
-        assert_close(out.float().cpu(), base.double() + ssum, tol, what + " accumulate")
-        out = run(base.to(dev).to(dtype).clone(), accumulate=True, relu_of=actd)
-        exp = torch.where(act > 0, base.double() + ssum, torch.zeros((), dtype=torch.float64))
-        assert_close(out.float().cpu(), exp, tol, what + " accumulate + gate")
-        assert bool((out.float().cpu()[act <= 0] == 0).all())
-        out = run(None, relu_of=actd)
-        exp = torch.where(act > 0, ssum, torch.zeros((), dtype=torch.float64))
-        assert_close(out.float().cpu(), exp, tol, what + " gate only")
 
 
 # ---------------------------------------------------------------------------------------- K4
@@ -441,93 +395,3 @@ def test_score_topk_float_and_sharded(dev):
     parts = [trg.score_topk(q.to(dev), cat[a:b].to(dev).contiguous(), 10, id_offset=a) for a, b in bounds]
     mv, mi = trg.topk_merge(torch.cat([x[0] for x in parts], 1), torch.cat([x[1] for x in parts], 1), 3, 10)
     assert torch.equal(mv, gv) and torch.equal(mi, gi)
-
-
-# ------------------------------------------------------------- fp32 sum rows / row finish (multi-GPU path)
-@pytest.mark.parametrize("f,long_rows", [(128, False), (256, False), (64, False), (16, False), (128, True)])
-def test_gather_fp32_output_rows_for_bf16_tables(dev, f, long_rows, monkeypatch):
-    """out_dtype = fp32 with a bf16 table (the partial sums a multi-GPU run reduces across ranks): the rows
-    are the UNROUNDED fp32 accumulations -- 1e-5 against an fp64 sum of the bf16 inputs, where the bf16
-    output would only be good to 4e-3 -- including accumulate and the long-row combine."""
-    if long_rows:
-        from truth_recommendation_gnn_b200 import graph as G
-        monkeypatch.setattr(G, "LONG_ROW_THRESHOLD", 64)
-    x, ei = _agg_case(300, 200, 6000, f, 5 + f, skew=True)
-    xb = x.bfloat16()
-    gen = torch.Generator().manual_seed(3)
-    coef = torch.randn(6000, generator=gen)
-    csr = trg.RelationGraph(ei.to(dev), 300, 200).fwd
-    s_plain = torch.zeros(200, f, dtype=torch.float64).index_add_(0, ei[1], xb.double()[ei[0]])
-    s_coef = torch.zeros(200, f, dtype=torch.float64).index_add_(0, ei[1], coef.double()[:, None] * xb.double()[ei[0]])
-    out = Fn.sage_agg_bwd(csr, None, xb.to(dev), out_dtype=torch.float32)
-    assert out.dtype == torch.float32
-    assert_close(out.cpu(), s_plain, TOL_F32, "fp32 sum rows of a bf16 table")
-    Fn.gather_wsum(csr, coef.to(dev), xb.to(dev), out=out, accumulate=True)           # accumulates in fp32
-    assert_close(out.cpu(), s_plain + s_coef, TOL_F32, "fp32 rows, accumulate")
-    rounded = Fn.sage_agg_bwd(csr, None, xb.to(dev))
-    assert rounded.dtype == torch.bfloat16
-    assert_close(rounded.float().cpu(), s_plain, TOL_BF16, "bf16 rows")
-    with pytest.raises(trg._lib.TrgError):
-        Fn.sage_agg_bwd(csr, None, x.to(dev), out_dtype=torch.bfloat16)               # only bf16 -> fp32 exists
-
-
-@pytest.mark.parametrize("dtype,in_f32", [(torch.float32, True), (torch.bfloat16, True), (torch.bfloat16, False)])
-def test_rows_finish(dev, dtype, in_f32):
-    """trg_rows_finish: out = gate(row_scale * in + add), fp32 arithmetic, one rounding."""
-    gen = torch.Generator().manual_seed(1)
-    n, f = 1000, 128
-    x = torch.randn(n, f, generator=gen)
-    x = x if in_f32 else x.bfloat16().float()
-    add = torch.randn(n, f, generator=gen).to(dtype).float()
-    act = torch.relu(torch.randn(n, f, generator=gen)).to(dtype).float()
-    rs = torch.rand(n, generator=gen)
-    xd = x.to(dev) if in_f32 else x.to(dev).to(dtype)
-    tol = TOL_F32 if dtype == torch.float32 else 2.0 ** -8          # one bf16 rounding of the result
-    out = Fn.rows_finish(xd, dtype, row_scale=rs.to(dev))
-    assert out.dtype == dtype
-    assert_close(out.float().cpu(), x.double() * rs.double()[:, None], tol, "row scale")
-    out = Fn.rows_finish(xd, dtype, add=add.to(dev).to(dtype), relu_of=act.to(dev).to(dtype))
-    exp = torch.where(act > 0, x.double() + add.double(), torch.zeros((), dtype=torch.float64))
-    assert_close(out.float().cpu(), exp, tol, "add + gate")
-    assert bool((out.float().cpu()[act <= 0] == 0).all())
-    if dtype == torch.float32:
-        assert torch.equal(out.cpu(), torch.where(act > 0, x + add, torch.zeros(())))    # exactly torch's fp32
-    assert Fn.rows_finish(xd[:0], dtype).shape == (0, f)
-
-
-@pytest.mark.parametrize("dtype,in_f32", [(torch.float32, True), (torch.bfloat16, True), (torch.bfloat16, False)])
-@pytest.mark.parametrize("n_peers", [1, 2, 3, 4, 8])
-def test_peer_reduce_rows(dev, dtype, in_f32, n_peers):
-    """trg_peer_reduce_rows = reduce-scatter + trg_rows_finish in one kernel: the owned row range of G partial
-    tables summed in rank order (bit-equal to the sequential fp32 sum), then 1/deg, local term, ReLU gate, one
-    rounding.  The G tables live on this device here; over NVLink they are the peers' mapped buffers."""
-    gen = torch.Generator().manual_seed(7 + n_peers)
-    rows, f, row0, n = 900, 128, 300, 500
-    parts = [torch.randn(rows, f, generator=gen) for _ in range(n_peers)]
-    if not in_f32:
-        parts = [p.bfloat16().float() for p in parts]
-    add = torch.randn(n, f, generator=gen).to(dtype).float()
-    act = torch.relu(torch.randn(n, f, generator=gen)).to(dtype).float()
-    rs = torch.rand(n, generator=gen)
-    pd = [p.to(dev) if in_f32 else p.to(dev).to(dtype) for p in parts]
-    seq = parts[0][row0:row0 + n].clone()
-    for p in parts[1:]:
-        seq = seq + p[row0:row0 + n]                       # fp32, rank order
-    out = Fn.peer_reduce_rows(pd, row0, n, dtype, row_scale=rs.to(dev))
-    assert out.dtype == dtype and out.shape == (n, f)
-    exp = seq * rs[:, None]
-    if dtype == torch.float32:
-        assert torch.equal(out.cpu(), exp)
-    else:
-        assert torch.equal(out.cpu(), exp.to(dtype))
-    out = Fn.peer_reduce_rows(pd, row0, n, dtype, add=add.to(dev).to(dtype), relu_of=act.to(dev).to(dtype))
-    exp = torch.where(act > 0, seq + add, torch.zeros(()))
-    assert torch.equal(out.cpu(), exp.to(dtype))
-    # same result as the two-step form it replaces
-    two = Fn.rows_finish(torch.stack([p[row0:row0 + n].float() for p in pd]).sum(0) if n_peers > 2 else
-                         (pd[0][row0:row0 + n].float() + (pd[1][row0:row0 + n].float() if n_peers == 2 else 0)),
-                         dtype, add=add.to(dev).to(dtype), relu_of=act.to(dev).to(dtype))
-    tol = TOL_F32 if dtype == torch.float32 else 2.0 ** -7
-    assert_close(out.float().cpu(), two.float().cpu(), tol, "fused vs reduce + finish")
-    assert Fn.peer_reduce_rows(pd, 0, 0, dtype).shape == (0, f)
-
