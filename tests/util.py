@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests (tolerances are BASELINE.json's north_star)."""
+import math
 import os
 
 import torch
@@ -10,6 +11,8 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 TOL_F32 = 1e-5   # relative, fp32 embeddings / losses / scores
 TOL_BF16 = 1e-2  # relative, bf16 storage with fp32 accumulation
+U = 2.0 ** -24    # fp32 unit roundoff
+BF16 = torch.bfloat16
 
 
 def load_golden(name):
@@ -129,3 +132,65 @@ def oracle_grads_bf16(h, layers, sd, g, neg, fin=None):
                            neg, g.interaction_type_tensor.float(), g.num_users)
     loss.backward()
     return {n: p.grad.float() for n, p in m.named_parameters()}
+
+
+# ------------------------------------------------------------------------------------------------
+# kernel-level tests: guarded buffers and element-wise checks
+# ------------------------------------------------------------------------------------------------
+def _bits(t):
+    return t.view(torch.int32 if t.element_size() == 4 else torch.int16)
+
+
+class Guarded:
+    """A [shape] output viewed inside a NaN-filled buffer with guard regions before and after it."""
+
+    def __init__(self, shape, dtype, dev, fill=None):
+        numel = math.prod(shape)
+        self.lead = 64                                 # 16-byte aligned for both dtypes
+        tail = 64 * (shape[-1] if len(shape) > 1 else 1) + 64
+        self.buf = torch.full((self.lead + numel + tail,), float("nan"), dtype=dtype, device=dev)
+        self.view = self.buf[self.lead:self.lead + numel].view(shape)
+        if fill is not None:
+            self.view.copy_(fill)
+        self.numel = numel
+        self.snap = self.buf.clone()
+
+    def check_guards(self, what):
+        b, s, e = _bits(self.buf), _bits(self.snap), self.lead + self.numel
+        assert torch.equal(b[:self.lead], s[:self.lead]), f"{what}: wrote before the output"
+        assert torch.equal(b[e:], s[e:]), f"{what}: wrote past the output"
+
+
+def nan_padded(x, dev, extra=67):
+    """``x`` on the device as the prefix view of a buffer whose remaining rows are NaN."""
+    big = torch.full((x.shape[0] + extra, *x.shape[1:]), float("nan"), dtype=x.dtype, device=dev)
+    big[:x.shape[0]] = x.to(dev)
+    return big[:x.shape[0]]
+
+
+def assert_bits(got, want, what):
+    got = got.detach().cpu()
+    assert got.dtype == want.dtype and got.shape == want.shape, (what, got.dtype, got.shape, want.shape)
+    bad = ~((got == want) | (torch.isnan(got) & torch.isnan(want)))
+    if bool(bad.any()):
+        idx = tuple(int(i) for i in bad.nonzero()[0])
+        raise AssertionError(f"{what}: {int(bad.sum())} of {got.numel()} entries differ (first at {idx}: got "
+                             f"{float(got[idx])!r}, want {float(want[idx])!r})")
+
+
+def check_bound(out, ref, absr, steps, out_dtype, what):
+    """|out - ref| <= steps 2^-24 absr (+ 2^-8 |ref| after a bf16 rounding), element by element; ``steps``
+    is per row."""
+    out = out.detach().double().cpu()
+    assert bool(torch.isfinite(out).all()), f"{what}: non-finite output"
+    bound = steps.double()[:, None] * U * absr
+    if out_dtype == BF16:
+        bound = bound * (1 + 2.0 ** -8) + 2.0 ** -8 * ref.abs()       # bf16 unit roundoff: 8-bit significand
+    err = (out - ref).abs()
+    bad = err > bound
+    if bool(bad.any()):
+        ratio = float((err / bound.clamp(min=1e-300)).max())
+        idx = tuple(int(i) for i in bad.nonzero()[0])
+        raise AssertionError(f"{what}: {int(bad.sum())} of {out.numel()} entries out of bound (worst err/bound "
+                             f"{ratio:.3g}; first at {idx}: got {float(out[idx])!r}, want {float(ref[idx])!r} "
+                             f"+- {float(bound[idx]):.3g})")

@@ -60,12 +60,16 @@ __global__ void __launch_bounds__(kThreads, VPL == 1 ? 3 : 2) edge_bce(const Bce
   constexpr int kUnroll = (LPR < 8 ? (LPR >= 4 ? 2 : 1) : (VPL == 1 ? 4 : 2)) * (TWO ? 1 : 2);
   static_assert(R < LPR, "row boundaries are held one per lane");
   __shared__ double red[2][kThreads / 32];
+  // fp64 running sums of this thread's fp32 loss terms, folded in once per chunk: one row group may walk a
+  // hub row of millions of edges, whose terms a single fp32 sum would carry ~1e-4 off
+  __shared__ double lane_sum[2][kThreads];
   const int lane = threadIdx.x & 31;
   const int gl = lane & (LPR - 1);
   const unsigned gmask = LPR == 32 ? 0xffffffffu : (((1u << LPR) - 1u) << (lane & ~(LPR - 1)));
   const int64_t r0 = ((int64_t)blockIdx.x * (kThreads / LPR) + threadIdx.x / LPR) * R;
   const bool want_grad = a.g_u != nullptr;
   float sp_sum = 0.f, sn_sum = 0.f;
+  lane_sum[0][threadIdx.x] = lane_sum[1][threadIdx.x] = 0.0;   // thread-private slots: no barrier
 
   if (r0 < a.n_users) {
     const int nr = (int)((a.n_users - r0) < (int64_t)R ? (a.n_users - r0) : (int64_t)R);
@@ -252,6 +256,9 @@ __global__ void __launch_bounds__(kThreads, VPL == 1 ? 3 : 2) edge_bce(const Bce
         a.c_pos[id_cur] = my_cpos;
         if (TWO) a.c_neg[id_cur] = my_cneg;
       }
+      lane_sum[0][threadIdx.x] += (double)sp_sum;
+      lane_sum[1][threadIdx.x] += (double)sn_sum;
+      sp_sum = sn_sum = 0.f;
       e0 += LPR;
       cp_cur = cp_nxt; id_cur = id_nxt; cn_cur = cn_nxt;
       cp_nxt = cp_nn; id_nxt = id_nn;
@@ -260,7 +267,7 @@ __global__ void __launch_bounds__(kThreads, VPL == 1 ? 3 : 2) edge_bce(const Bce
   }
 
   // deterministic CTA reduction -> one (sp, sn) pair of doubles per CTA
-  double dsp = sp_sum, dsn = sn_sum;
+  double dsp = lane_sum[0][threadIdx.x], dsn = lane_sum[1][threadIdx.x];
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     dsp += __shfl_xor_sync(0xffffffffu, dsp, o);
@@ -315,12 +322,14 @@ __global__ void __launch_bounds__(kThreads, 3) edge_anchor_ring(const BceArgs a)
   constexpr unsigned full = 0xffffffffu;
   extern __shared__ __align__(16) unsigned char ring_raw[];
   __shared__ double red[2][kThreads / 32];
+  __shared__ double lane_sum[kThreads];   // fp64 running sum of the thread's fp32 loss terms (as in edge_bce)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint32_t ring_a = static_cast<uint32_t>(__cvta_generic_to_shared(ring_raw)) +
                           (uint32_t)(warp * S * 512 + lane * 16);
   const int64_t r0 = ((int64_t)blockIdx.x * (kThreads / 32) + warp) * R;
   const bool want_grad = a.g_u != nullptr;
   float s_sum = 0.f;
+  lane_sum[threadIdx.x] = 0.0;
 
   if (r0 < a.n_users) {
     const int nr = (int)((a.n_users - r0) < (int64_t)R ? (a.n_users - r0) : (int64_t)R);
@@ -450,6 +459,8 @@ __global__ void __launch_bounds__(kThreads, 3) edge_anchor_ring(const BceArgs a)
         t += bsz;
       }
       if (want_grad && lane < cnt) a.c_pos[my_id] = my_c;
+      lane_sum[threadIdx.x] += (double)s_sum;
+      s_sum = 0.f;
       __syncwarp();           // every lane is done with this group's slots: refill them two groups ahead
       const int nid_next = load_id(e_base + 3 * G);
       issue(e_base + 2 * G, nid, slot);
@@ -461,7 +472,7 @@ __global__ void __launch_bounds__(kThreads, 3) edge_anchor_ring(const BceArgs a)
   }
 
   // deterministic CTA reduction -> one (sp, sn) pair of doubles per CTA (layout of edge_bce)
-  double dsum = s_sum;
+  double dsum = lane_sum[threadIdx.x];
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) dsum += __shfl_xor_sync(0xffffffffu, dsum, o);
   if (lane == 0) red[0][warp] = dsum;
@@ -562,6 +573,10 @@ extern "C" int trg_edge_bce_fwd(const int32_t* rowptr_u, const int32_t* col_p, c
   TRG_CHECK_ARG(dtype == TRG_F32 || dtype == TRG_BF16, "trg_edge_bce_fwd: unknown dtype %d", dtype);
   TRG_CHECK_ARG(hidden > 0 && (hidden * es) % 16 == 0,
                 "trg_edge_bce_fwd: row width %d x %d bytes is not a multiple of 16 bytes", hidden, es);
+  if ((int64_t)hidden * es > 1024) {   // checked here, not at dispatch, so n_users = 0 is refused alike
+    set_error("trg_edge_bce_fwd: rows wider than 1024 bytes are not supported (%d x %d bytes)", hidden, es);
+    return TRG_E_UNSUPPORTED;
+  }
   if (workspace == nullptr || workspace_bytes < trg_edge_bce_workspace_bytes(n_users)) {
     set_error("trg_edge_bce_fwd: workspace %zu < required %zu", workspace_bytes,
               trg_edge_bce_workspace_bytes(n_users));
@@ -606,6 +621,10 @@ extern "C" int trg_edge_anchor_loss(const int32_t* rowptr, const int32_t* col, c
   const int es = dtype == TRG_BF16 ? 2 : 4;
   TRG_CHECK_ARG(hidden > 0 && (hidden * es) % 16 == 0,
                 "trg_edge_anchor_loss: row width %d x %d bytes is not a multiple of 16 bytes", hidden, es);
+  if ((int64_t)hidden * es > 1024) {   // checked here, not at dispatch, so n_rows = 0 is refused alike
+    set_error("trg_edge_anchor_loss: rows wider than 1024 bytes are not supported (%d x %d bytes)", hidden, es);
+    return TRG_E_UNSUPPORTED;
+  }
   if (workspace == nullptr || workspace_bytes < trg_edge_bce_workspace_bytes(n_rows)) {
     set_error("trg_edge_anchor_loss: workspace %zu < required %zu", workspace_bytes,
               trg_edge_bce_workspace_bytes(n_rows));
